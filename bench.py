@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the B200-native InstructAny2Pix denoising hot path.
 
-    python bench.py --gpus N --steps K --warmup W [--workload c3|c2|c4|b1|c1] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--workload c3|c2|c4|b1|c1] [--impl reference] [--dump-outputs DIR]
 
 A "step" is ONE complete 50-step DDIM + CFG sampling trajectory for the per-GPU batch (the unit of BASELINE.json's
 metric, images/sec at 1024^2): 50 x (CUDA-graph replay of the SDXL-class UNet at CFG batch 2B + fused CFG/DDIM kernel),
@@ -18,6 +18,10 @@ sample, warmed once), "gpu_eager_baseline" (the reference-equivalent PyTorch eag
 the same GPU, cuDNN / cuBLAS / SDPA -- one CFG UNet step, N = 1 only), "e2e" (whole request batches through the public API and
 ``parallel.run_sharded``: pinned-host inputs -> device, trajectory, VAE decode, ordered gather of every rank's images on rank 0
 (NCCL), device -> host; ``first_batch_sha256`` is identical for every GPU count).
+
+--dump-outputs DIR writes what the last timed step returned to its caller (rank 0) as DIR/<name>.npy in float32: "latents" of
+the device-resident trajectory and "e2e_images" of the last end-to-end batch (c1: "embedding" and "e2e_embedding").  Weights
+and inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -108,6 +112,22 @@ class ClockSampler:
                 if v.lower().startswith("active"):
                     reasons.add(name)
         return dict(sm_mhz=statistics.median(sm) if sm else None, sm_max_mhz=mx, reasons=sorted(reasons), samples=len(sm))
+
+
+DUMP_MAX_ELEMS = 1 << 22          # float32 elements per dumped array (16 MB): the two arrays of a run stay well under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor as ``out_dir/<name>.npy`` in float32.  A tensor of more than DUMP_MAX_ELEMS elements is replaced by a
+    sample of its flattened elements at fixed (seeded, ascending) indices, the same on every run."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().to("cpu", torch.float32)
+        if t.numel() > DUMP_MAX_ELEMS:
+            idx = torch.randint(t.numel(), (DUMP_MAX_ELEMS,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.numpy())
 
 
 # ------------------------------------------------------------------------------------------------ model + inputs
@@ -484,7 +504,7 @@ def bench_prior(args, wl, dev, rank, world, local):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        prior.generate_diffusion(3, 0, src_d, device=dev, **kw)       # noise drawn on the device, result stays there
+        emb, _ = prior.generate_diffusion(3, 0, src_d, device=dev, **kw)       # noise drawn on the device, result stays there
     e1.record()
     sync_all()
     clk = clocks.stop()
@@ -527,6 +547,8 @@ def bench_prior(args, wl, dev, rank, world, local):
         ms, ms_e2e = tt.tolist()
     if rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(embedding=emb, e2e_embedding=y))
     pk = peaks()
     ms_step = ms / args.steps
     step_us = ms_step * 1e3 / PRIOR_STEPS
@@ -569,7 +591,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-eager-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the b200 implementation")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         return reference_arm(args, wl)
@@ -629,7 +656,7 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        run_trajectory(hot, dev_in, NS)
+        lat = run_trajectory(hot, dev_in, NS)
     e1.record()
     sync_all()
     clk = clocks.stop()
@@ -678,6 +705,8 @@ def main():
         return
     d2h = res.numel() * res.element_size() / args.steps
     sha = hashlib.sha256(res[:B].numpy().tobytes()).hexdigest()[:16]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(latents=lat, e2e_images=res[-B:]))
 
     pk = peaks()
     ms_step = ms / args.steps
