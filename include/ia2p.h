@@ -25,7 +25,9 @@ extern "C" {
 
 enum { IA2P_F32 = 0, IA2P_BF16 = 1, IA2P_F16 = 2 };
 enum { IA2P_E_ARG = -1, IA2P_E_DEVICE = -2, IA2P_E_SHAPE = -3, IA2P_E_ALIGN = -4, IA2P_E_DRIVER = -5 };
-enum { IA2P_EPI_NONE = 0, IA2P_EPI_GEGLU = 1 };
+/* GEMM epilogues.  GELU (exact erf, the GEGLU gate's evaluation) and QUICK_GELU (x * sigmoid(1.702 x), CLIP's quick_gelu) act on
+ * the LN-corrected accumulator plus bias; they need bf16 output and no residual / rowbias / LN-producer or column statistics. */
+enum { IA2P_EPI_NONE = 0, IA2P_EPI_GEGLU = 1, IA2P_EPI_GELU = 2, IA2P_EPI_QUICK_GELU = 3 };
 enum { IA2P_ACT_NONE = 0, IA2P_ACT_GELU_NEW = 1, IA2P_ACT_SILU = 2 };
 
 int ia2p_version(void);
@@ -105,6 +107,14 @@ int64_t ia2p_groupnorm_workspace_bytes(int64_t batch, int groups);
  * [prior].  Replaces [3P] BasicTransformerBlock.norm1/2/3 and GPT-2 ln_1/ln_2/ln_f.  cols % 8 == 0, cols <= 2048. */
 int ia2p_layernorm(const void* x, int x_dtype, const float* gamma, const float* beta, void* y, int y_dtype,
                    int64_t rows, int64_t cols, float eps, void* stream);
+
+/* CLIP text embeddings: out[r] = tok[ids[r]] + pos[r % T], fp32 [n*T, C] (the residual stream).  Replaces [3P] CLIPTextEmbeddings
+ * (token_embedding + position_embedding, default position_ids).  ids int64 [n, T]; tok bf16 [V, C]; pos fp32 [P >= T, C].
+ * An id outside [0, V) reads nothing and yields a NaN row.  out_bf16 / stats (nullable, together): the bf16 copy and per-row
+ * (sum, sum of squares), stats [n*T][1][2]: the producer format of ia2p_gemm_ln_bf16, so layer 0's layer_norm1 folds into the QKV
+ * GEMM like every other LayerNorm.  C % 8 == 0. */
+int ia2p_clip_embed(const int64_t* ids, int64_t n, int64_t T, const void* tok, int64_t V, const float* pos, int64_t P,
+                    int64_t C, float* out, void* out_bf16, float* stats, void* stream);
 
 /* ---------------------------------------------------------------- tcgen05 GEMM / implicit-GEMM conv (tensor-bound) */
 
@@ -224,6 +234,15 @@ int ia2p_softmax_rows_f32_bf16(const float* scores, int64_t ld, void* out, int64
 int ia2p_flash_self_attn_bf16(const void* q, const void* k, const void* v, int64_t ld,
                               void* out, int64_t ldo, int64_t batch, int64_t n_tokens, int heads,
                               float softmax_scale, void* stream);
+
+/* Causal self-attention for short sequences, head_dim 64: key j is masked for query i when j > i (no padding mask: CLIP attends
+ * over pad tokens causally).  Replaces CLIPAttention with its causal mask ([3P] transformers CLIPTextTransformer, reached through
+ * StableDiffusionXLPipeline.encode_prompt at ip_adapter.py:320-342 and the refiner at pipeline.py:358-361).  Same operand layout
+ * as ia2p_flash_self_attn_bf16 (q/k/v: strided views of one fused [n*T, 3C] QKV output); fp32 softmax, masked keys contribute
+ * exactly 0.  1 <= T <= 128; q/k/v/out 16-byte aligned. */
+int ia2p_causal_self_attn_bf16(const void* q, const void* k, const void* v, int64_t ld,
+                               void* out, int64_t ldo, int64_t n, int64_t T, int heads,
+                               float softmax_scale, void* stream);
 
 /* Decoupled cross-attention: out = softmax(Q Kt^T) Vt + ip_scale * softmax(Q Ki^T) Vi in ONE kernel.
  * Replaces the two SDPA calls + add at attention_processor.py:371-373,387-389,397.

@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("IA2P_LIB_OVERRIDE") or os.path.join(_HERE, "libia2p_sm100a.so")   # override: A/B experiment builds only
 
 F32, BF16, F16 = 0, 1, 2
-EPI_NONE, EPI_GEGLU = 0, 1
+EPI_NONE, EPI_GEGLU, EPI_GELU, EPI_QUICK_GELU = 0, 1, 2, 3
 ACT_NONE, ACT_GELU_NEW, ACT_SILU = 0, 1, 2
 
 _p, _i, _l, _f = C.c_void_p, C.c_int, C.c_int64, C.c_float
@@ -35,6 +35,7 @@ SIGNATURES = {
     "ia2p_groupnorm_nhwc": ([_p, _l, _p, _l, _i, _p, _p, _p, _p, _l, _l, _i, _f, _i, _p, _l, _p, _l, _p, _p], _i),
     "ia2p_groupnorm_workspace_bytes": ([_l, _i], _l),
     "ia2p_layernorm": ([_p, _i, _p, _p, _p, _i, _l, _l, _f, _p], _i),
+    "ia2p_clip_embed": ([_p, _l, _l, _p, _l, _p, _l, _l, _p, _p, _p, _p], _i),
     "ia2p_gemm_bf16": ([_p, _l, _l, _p, _l, _l, _p, _p, _l, _l, _l, _p, _p, _l, _p, _l, _i, _i, _i, _p], _i),
     "ia2p_gemm_ln_bf16": ([_p, _l, _l, _p, _l, _l, _p, _p, _l, _l, _l, _p, _p, _l, _p, _l, _i, _i, _i,
                            _p, _l, _p, _p, _p, _l, _p, _f, _p], _i),
@@ -54,6 +55,7 @@ SIGNATURES = {
     "ia2p_conv1x1_nchw_small": ([_p, _p, _p, _p, _l, _l, _l, _l, _f, _p], _i),
     "ia2p_softmax_rows_f32_bf16": ([_p, _l, _p, _l, _l, _l, _f, _p], _i),
     "ia2p_flash_self_attn_bf16": ([_p, _p, _p, _l, _p, _l, _l, _l, _i, _f, _p], _i),
+    "ia2p_causal_self_attn_bf16": ([_p, _p, _p, _l, _p, _l, _l, _l, _i, _f, _p], _i),
     "ia2p_decoupled_cross_attn_bf16": ([_p, _l, _p, _p, _l, _i, _p, _p, _l, _i, _f, _p, _l, _l, _l, _i, _f, _p], _i),
     "ia2p_gemm_smallm": ([_p, _l, _p, _p, _p, _l, _p, _l, _l, _l, _l, _i, _i, _p], _i),
     "ia2p_causal_attn_small_f32": ([_p, _p, _l, _l, _i, _p], _i),

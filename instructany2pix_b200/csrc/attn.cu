@@ -349,6 +349,131 @@ static int launch_cross(const void* q, int64_t ldq, const void* kt, const void* 
   return 0;
 }
 
+// ================================================================ causal self-attention, T <= 128 (CLIP text towers)
+// One CTA per (head, sequence) holds the whole sequence: Q, K, V padded to TK rows (multiple of 16, zero-filled) in smem.  Warp w
+// owns query rows [16w, 16w + 16) and, causally, only the key tiles [0, 16w + 16): the MMAs past the diagonal are skipped.  Keys
+// j > i are set to -inf before the exponentials (exactly 0 after them), the softmax is fp32 over the whole row at once (all keys
+// are resident: no online rescaling), P is normalised before the bf16 pack.  mma.sync rather than tcgen05: a 77-token head is
+// 5 x 16 query rows, far below one 128-row UMMA tile, and the whole problem of a CFG pair (2 x 20 heads) is 40 CTAs.
+template <int TK>
+__global__ void __launch_bounds__(TK * 2)
+causal_self_attn_kernel(const __nv_bfloat16* __restrict__ q, const __nv_bfloat16* __restrict__ k,
+                        const __nv_bfloat16* __restrict__ v, long long ld, __nv_bfloat16* __restrict__ out, long long ldo,
+                        int T, float scale_log2) {
+  pdl_launch_dependents();   // programmatic dependent launch: see common.cuh
+  pdl_wait();
+  constexpr int NT = TK / 8;
+  extern __shared__ __align__(128) uint8_t smem[];
+  const uint32_t sQ = smem_u32(smem);        // TK x 64 each
+  const uint32_t sK = sQ + TK * 128;
+  const uint32_t sV = sK + TK * 128;
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int g = lane >> 2, t = lane & 3;
+  const int h = blockIdx.x;
+  const long long tok0 = (long long)blockIdx.y * T;
+  load_tile(sQ, q + tok0 * ld + h * 64, ld, TK, T, tid, TK * 2);
+  load_tile(sK, k + tok0 * ld + h * 64, ld, TK, T, tid, TK * 2);
+  load_tile(sV, v + tok0 * ld + h * 64, ld, TK, T, tid, TK * 2);
+  cp_async_commit();
+  cp_async_wait<0>();
+  __syncthreads();
+  const int r0 = warp * 16;
+  if (r0 >= T) return;                        // no barrier follows
+
+  uint32_t qf[4][4];
+#pragma unroll
+  for (int kk = 0; kk < 4; ++kk) {
+    const int r = r0 + (lane & 7) + ((lane >> 3) & 1) * 8;
+    ldsm_x4(sQ + tile_off(r, kk * 2 + (lane >> 4)), qf[kk][0], qf[kk][1], qf[kk][2], qf[kk][3]);
+  }
+  float s[NT][4];
+#pragma unroll
+  for (int nt = 0; nt < NT; ++nt) {
+    s[nt][0] = s[nt][1] = s[nt][2] = s[nt][3] = 0.f;
+    if (nt < 2 * warp + 2) {                  // warp-uniform: key tiles at or left of the diagonal
+#pragma unroll
+      for (int kp = 0; kp < 2; ++kp) {
+        uint32_t b0, b1, b2, b3;
+        ldsm_x4(sK + tile_off(nt * 8 + (lane & 7), kp * 4 + (lane >> 3)), b0, b1, b2, b3);
+        mma_bf16(s[nt], qf[kp * 2], b0, b1);
+        mma_bf16(s[nt], qf[kp * 2 + 1], b2, b3);
+      }
+    }
+  }
+  const int row0 = r0 + g, row1 = row0 + 8;
+  float mx0 = -INFINITY, mx1 = -INFINITY;
+#pragma unroll
+  for (int nt = 0; nt < NT; ++nt) {
+#pragma unroll
+    for (int e = 0; e < 2; ++e) {
+      const int key = nt * 8 + 2 * t + e;
+      s[nt][e] = key <= row0 ? s[nt][e] * scale_log2 : -INFINITY;
+      s[nt][2 + e] = key <= row1 ? s[nt][2 + e] * scale_log2 : -INFINITY;
+      mx0 = fmaxf(mx0, s[nt][e]);
+      mx1 = fmaxf(mx1, s[nt][2 + e]);
+    }
+  }
+  mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 1)); mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 2));
+  mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 1)); mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 2));
+  float l0 = 0.f, l1 = 0.f;                   // key 0 is never masked: the row maxima are finite
+#pragma unroll
+  for (int nt = 0; nt < NT; ++nt) {
+    s[nt][0] = ex2_approx(s[nt][0] - mx0); s[nt][1] = ex2_approx(s[nt][1] - mx0);
+    s[nt][2] = ex2_approx(s[nt][2] - mx1); s[nt][3] = ex2_approx(s[nt][3] - mx1);
+    l0 += s[nt][0] + s[nt][1];
+    l1 += s[nt][2] + s[nt][3];
+  }
+  l0 += __shfl_xor_sync(0xffffffffu, l0, 1); l0 += __shfl_xor_sync(0xffffffffu, l0, 2);
+  l1 += __shfl_xor_sync(0xffffffffu, l1, 1); l1 += __shfl_xor_sync(0xffffffffu, l1, 2);
+  const float i0 = 1.f / l0, i1 = 1.f / l1;
+  float o[8][4];
+#pragma unroll
+  for (int i = 0; i < 8; ++i) o[i][0] = o[i][1] = o[i][2] = o[i][3] = 0.f;
+#pragma unroll
+  for (int kk = 0; kk < TK / 16; ++kk) {
+    if (kk <= warp) {                         // 16-key steps at or left of the diagonal
+      uint32_t pa[4];
+      pa[0] = pack_bf16x2(s[2 * kk][0] * i0, s[2 * kk][1] * i0);
+      pa[1] = pack_bf16x2(s[2 * kk][2] * i1, s[2 * kk][3] * i1);
+      pa[2] = pack_bf16x2(s[2 * kk + 1][0] * i0, s[2 * kk + 1][1] * i0);
+      pa[3] = pack_bf16x2(s[2 * kk + 1][2] * i1, s[2 * kk + 1][3] * i1);
+#pragma unroll
+      for (int dp = 0; dp < 4; ++dp) {
+        uint32_t b0, b1, b2, b3;
+        const int r = kk * 16 + (lane & 7) + ((lane >> 3) & 1) * 8;
+        ldsm_x4_t(sV + tile_off(r, dp * 2 + (lane >> 4)), b0, b1, b2, b3);
+        mma_bf16(o[2 * dp], pa, b0, b1);
+        mma_bf16(o[2 * dp + 1], pa, b2, b3);
+      }
+    }
+  }
+  // stage this warp's 16 x 64 tile through its own (consumed) rows of the Q tile for 16-byte coalesced stores
+  __syncwarp();
+#pragma unroll
+  for (int dt = 0; dt < 8; ++dt) {
+    *reinterpret_cast<uint32_t*>(smem + tile_off(row0, dt) + t * 4) = pack_bf16x2(o[dt][0], o[dt][1]);
+    *reinterpret_cast<uint32_t*>(smem + tile_off(row1, dt) + t * 4) = pack_bf16x2(o[dt][2], o[dt][3]);
+  }
+  __syncwarp();
+  __nv_bfloat16* og = out + tok0 * ldo + h * 64;
+  for (int id = lane; id < 16 * 8; id += 32) {
+    const int r = r0 + (id >> 3), ch = id & 7;
+    if (r < T) *reinterpret_cast<uint4*>(og + (long long)r * ldo + ch * 8) = *reinterpret_cast<const uint4*>(smem + tile_off(r, ch));
+  }
+}
+
+template <int TK>
+static int launch_causal(const void* q, const void* k, const void* v, int64_t ld, void* out, int64_t ldo, int64_t n, int64_t T,
+                         int heads, float scale, cudaStream_t st) {
+  constexpr int smem = 3 * TK * 128;
+  IA2P_ONCE_PER_DEVICE(IA2P_CUDA(cudaFuncSetAttribute(causal_self_attn_kernel<TK>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)));
+  launch_pdl(causal_self_attn_kernel<TK>, dim3((unsigned)heads, (unsigned)n), dim3(TK * 2), smem, st,
+             static_cast<const __nv_bfloat16*>(q), static_cast<const __nv_bfloat16*>(k), static_cast<const __nv_bfloat16*>(v), ld,
+             static_cast<__nv_bfloat16*>(out), ldo, (int)T, scale * kLog2e);
+  IA2P_LAUNCH_CHECK();
+  return 0;
+}
+
 }  // namespace ia2p
 
 namespace ia2p {
@@ -386,6 +511,21 @@ extern "C" int ia2p_flash_self_attn_bf16(const void* q, const void* k, const voi
       static_cast<__nv_bfloat16*>(out), ldo, (int)n_tokens, softmax_scale * kLog2e);
   IA2P_LAUNCH_CHECK();
   return 0;
+}
+
+extern "C" int ia2p_causal_self_attn_bf16(const void* q, const void* k, const void* v, int64_t ld, void* out, int64_t ldo,
+                                          int64_t n, int64_t T, int heads, float softmax_scale, void* stream) {
+  IA2P_REQUIRE(q && k && v && out && n > 0 && heads > 0, IA2P_E_ARG, "causal_self_attn: bad arguments");
+  IA2P_REQUIRE(T >= 1 && T <= 128, IA2P_E_SHAPE, "causal_self_attn: T=%lld must be in [1, 128]", (long long)T);
+  IA2P_REQUIRE(heads <= 65535 && n <= 65535, IA2P_E_SHAPE, "causal_self_attn: heads/n too large");
+  IA2P_REQUIRE(ld % 8 == 0 && ldo % 8 == 0 && ((reinterpret_cast<uintptr_t>(q) | reinterpret_cast<uintptr_t>(k) |
+               reinterpret_cast<uintptr_t>(v) | reinterpret_cast<uintptr_t>(out)) & 15) == 0,
+               IA2P_E_ALIGN, "causal_self_attn: ld/ldo must be multiples of 8 and q/k/v/out 16-byte aligned");
+  if (int e = check_device()) return e;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (T <= 32) return launch_causal<32>(q, k, v, ld, out, ldo, n, T, heads, softmax_scale, st);
+  if (T <= 80) return launch_causal<80>(q, k, v, ld, out, ldo, n, T, heads, softmax_scale, st);
+  return launch_causal<128>(q, k, v, ld, out, ldo, n, T, heads, softmax_scale, st);
 }
 
 extern "C" int ia2p_decoupled_cross_attn_bf16(const void* q, int64_t ldq, const void* k_text, const void* v_text, int64_t ldkv,

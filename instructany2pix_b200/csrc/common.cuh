@@ -96,6 +96,8 @@ __device__ __forceinline__ float gelu_erf_f(float v) {
   const float q = 0.5f * p * e;
   return v * (v >= 0.f ? 1.0f - q : q);
 }
+// CLIP's quick_gelu, v * sigmoid(1.702 v)
+__device__ __forceinline__ float quick_gelu_f(float v) { return v / (1.0f + __expf(-1.702f * v)); }
 __device__ __forceinline__ float gelu_new_f(float v) {
   return 0.5f * v * (1.0f + tanhf(0.79788456080286535588f * (v + 0.044715f * v * v * v)));
 }

@@ -83,6 +83,7 @@ struct TcParams {
   long long ldo, ldr;
   long long ost_x, ost_y, ost_b;   // EPI >= 1 output map: element strides of the pixel grid (0 -> dense: ldo, ldo*Wo, ldo*Wo*Ho)
   int geglu, out_f32, res_f32;
+  int act;                         // EPI 3 only: IA2P_EPI_GELU | IA2P_EPI_QUICK_GELU on (LN-corrected acc + bias), else 0
   // LayerNorm folding (DESIGN.md): a PRODUCER of the fp32 residual stream also emits a bf16 copy of its output rows and
   // per-row partial (sum, sum of squares) over each column half of every N tile; a CONSUMER multiplies the raw bf16 rows
   // by gamma-scaled weights and finishes LN in its epilogue: rstd[m] * (acc - mean[m] * c1[n]) + c2[n].
@@ -608,6 +609,13 @@ tc_gemm_kernel(const __grid_constant__ TcMaps maps, const __grid_constant__ TcPa
                 }
                 f[i] = fmaf(__uint_as_float(v[i]), ln_rstd, bv.x); f[i + 1] = fmaf(__uint_as_float(v[i + 1]), ln_rstd, bv.y);
                 f[i + 2] = fmaf(__uint_as_float(v[i + 2]), ln_rstd, bv.z); f[i + 3] = fmaf(__uint_as_float(v[i + 3]), ln_rstd, bv.w);
+              }
+              if (p.act == IA2P_EPI_GELU) {
+#pragma unroll
+                for (int i = 0; i < 32; ++i) f[i] = gelu_erf_f(f[i]);
+              } else if (p.act == IA2P_EPI_QUICK_GELU) {
+#pragma unroll
+                for (int i = 0; i < 32; ++i) f[i] = quick_gelu_f(f[i]);
               }
             } else {
               // GEGLU: accumulator columns come in 64-wide groups [32 value | 32 gate] (W rows interleaved, packing.interleave_geglu)
@@ -1622,6 +1630,10 @@ extern "C" int ia2p_gemm_ln_bf16(const void* A, int64_t lda, int64_t K1, const v
                IA2P_E_ALIGN, "gemm: fp32 residual must be 32-byte aligned with ldr%%8==0");
   const bool geglu = epilogue == IA2P_EPI_GEGLU;
   IA2P_REQUIRE(!geglu || (N % 64 == 0 && residual == nullptr && rowbias == nullptr && out_dtype == IA2P_BF16), IA2P_E_ARG, "gemm: GEGLU needs N%%64==0, bf16 output and no residual/rowbias");
+  const bool act = epilogue == IA2P_EPI_GELU || epilogue == IA2P_EPI_QUICK_GELU;
+  IA2P_REQUIRE(!act || (residual == nullptr && rowbias == nullptr && out_dtype == IA2P_BF16 && out_bf16 == nullptr &&
+                        stats_out == nullptr && colstats == nullptr), IA2P_E_ARG,
+               "gemm: GELU / quick-GELU epilogues need bf16 output and no residual, rowbias, LN statistics or column statistics");
   IA2P_REQUIRE(rowbias == nullptr || rows_per_batch > 0, IA2P_E_ARG, "gemm: rowbias needs rows_per_batch");
   IA2P_REQUIRE(M < (1ll << 31) && N < (1ll << 31), IA2P_E_SHAPE, "gemm: M/N too large");
 
@@ -1664,6 +1676,8 @@ extern "C" int ia2p_gemm_ln_bf16(const void* A, int64_t lda, int64_t K1, const v
   p.colstats = colstats;
   p.ln_stats = ln_stats; p.ln_c1 = ln_c1; p.ln_parts = (int)ln_parts;
   p.ln_inv_n = 1.0f / (float)(K1 + K2); p.ln_eps = ln_eps;
+  p.act = act ? epilogue : 0;
+  IA2P_REQUIRE(!act || tma_epilogue_bf16(p), IA2P_E_ARG, "gemm: GELU / quick-GELU epilogues need the bf16 TMA-store epilogue");
   return dispatch_tc(maps, p, bn, static_cast<cudaStream_t>(stream));
 }
 

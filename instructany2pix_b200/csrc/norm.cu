@@ -282,6 +282,44 @@ static int launch_ln(const void* x, const float* gamma, const float* beta, void*
   return 0;
 }
 
+// ---------------------------------------------------------------- CLIP token + position embedding (warp per row)
+// out[r] = tok[ids[r]] + pos[r % T] in fp32; an id outside [0, V) reads nothing and yields a NaN row.  Optionally the bf16 copy
+// and the row's (sum, sum of squares) in the producer format of ia2p_gemm_ln_bf16 (one part per row).
+__global__ void clip_embed_kernel(const long long* __restrict__ ids, const __nv_bfloat16* __restrict__ tok, long long V,
+                                  const float* __restrict__ pos, float* __restrict__ out, __nv_bfloat16* __restrict__ out_bf16,
+                                  float* __restrict__ stats, long long rows, int T, int cols) {
+  pdl_launch_dependents();   // programmatic dependent launch: see common.cuh
+  pdl_wait();
+  const int lane = threadIdx.x & 31;
+  const long long row = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
+  if (row >= rows) return;
+  const long long id = __ldg(ids + row);
+  const bool ok = id >= 0 && id < V;
+  const float* pr = pos + (row % T) * cols;
+  float s = 0.f, q = 0.f;
+  for (int v = lane; v < cols / 8; v += 32) {
+    float a[8], b[8];
+    if (ok) {
+      Vec8<__nv_bfloat16>::load(tok + id * cols + v * 8, a);
+      Vec8<float>::load(pr + v * 8, b);
+#pragma unroll
+      for (int j = 0; j < 8; ++j) a[j] += b[j];
+    } else {
+#pragma unroll
+      for (int j = 0; j < 8; ++j) a[j] = __int_as_float(0x7fffffff);
+    }
+#pragma unroll
+    for (int j = 0; j < 8; ++j) { s += a[j]; q = fmaf(a[j], a[j], q); }
+    Vec8<float>::store(out + row * cols + v * 8, a);
+    if (out_bf16 != nullptr) Vec8<__nv_bfloat16>::store(out_bf16 + row * cols + v * 8, a);
+  }
+  if (stats != nullptr) {
+    s = warp_sum(s);
+    q = warp_sum(q);
+    if (lane == 0) { stats[2 * row] = s; stats[2 * row + 1] = q; }
+  }
+}
+
 }  // namespace ia2p
 
 using namespace ia2p;
@@ -357,4 +395,23 @@ extern "C" int ia2p_layernorm(const void* x, int x_dtype, const float* gamma, co
   if (x_dtype == IA2P_F32 && y_dtype == IA2P_F32) return launch_ln<float, float>(x, gamma, beta, y, rows, cols, eps, st);
   set_error("layernorm: unsupported dtype pair (%d -> %d)", x_dtype, y_dtype);
   return IA2P_E_ARG;
+}
+
+extern "C" int ia2p_clip_embed(const int64_t* ids, int64_t n, int64_t T, const void* tok, int64_t V, const float* pos, int64_t P,
+                               int64_t C, float* out, void* out_bf16, float* stats, void* stream) {
+  IA2P_REQUIRE(ids && tok && pos && out && n > 0 && T > 0 && V > 0 && C > 0, IA2P_E_ARG, "clip_embed: bad arguments");
+  IA2P_REQUIRE((out_bf16 == nullptr) == (stats == nullptr), IA2P_E_ARG, "clip_embed: out_bf16 and stats must be given together");
+  IA2P_REQUIRE(T <= P, IA2P_E_SHAPE, "clip_embed: T=%lld exceeds the %lld positions of the table", (long long)T, (long long)P);
+  IA2P_REQUIRE(C % 8 == 0, IA2P_E_SHAPE, "clip_embed: C=%lld must be a multiple of 8", (long long)C);
+  IA2P_REQUIRE((reinterpret_cast<uintptr_t>(tok) & 15) == 0 && (reinterpret_cast<uintptr_t>(out_bf16) & 15) == 0 &&
+               (reinterpret_cast<uintptr_t>(pos) & 31) == 0 && (reinterpret_cast<uintptr_t>(out) & 31) == 0 &&
+               (reinterpret_cast<uintptr_t>(ids) & 7) == 0, IA2P_E_ALIGN, "clip_embed: misaligned table or output");
+  if (int e = check_device()) return e;
+  const long long rows = n * T;
+  const int block = 256;
+  launch_pdl(clip_embed_kernel, dim3((unsigned)((rows * 32 + block - 1) / block)), dim3(block), 0, static_cast<cudaStream_t>(stream),
+             reinterpret_cast<const long long*>(ids), static_cast<const __nv_bfloat16*>(tok), (long long)V, pos, out,
+             static_cast<__nv_bfloat16*>(out_bf16), stats, rows, (int)T, (int)C);
+  IA2P_LAUNCH_CHECK();
+  return 0;
 }

@@ -305,6 +305,32 @@ def layernorm(x, gamma, beta, eps, out_dtype=None):
     return out
 
 
+def clip_embed(ids, tok, pos, want_ln=False):
+    """CLIP token + position embedding: fp32 [n*T, C] = tok[ids] + pos[:T] (ids int64 [n, T], tok bf16 [V, C], pos fp32 [P, C]).
+    ``want_ln``: also the bf16 copy and per-row (sum, sum of squares) [n*T, 1, 2] that ``gemm(ln=...)`` folds LayerNorm with.
+    Ids on the host are range-checked here (then copied to the table's device); ids already on the device are not
+    (that would need a sync): an id outside [0, V) yields a NaN row."""
+    lib = _lib.load()
+    _need(tok, torch.bfloat16, "tok", 2)
+    assert tok.is_contiguous()
+    pos = _need(pos, torch.float32, "pos", 2).contiguous()
+    if ids.dtype != torch.int64 or ids.ndim != 2:
+        raise IA2PError(f"clip_embed: ids must be int64 [n, T], got {ids.dtype} {tuple(ids.shape)}")
+    V, C = tok.shape
+    if not ids.is_cuda:
+        if ids.numel() and (int(ids.min()) < 0 or int(ids.max()) >= V):
+            raise IA2PError(f"clip_embed: token ids outside [0, {V})")
+        ids = ids.to(tok.device)
+    ids = ids.contiguous()
+    n, T = ids.shape
+    out = torch.empty(n * T, C, device=tok.device, dtype=torch.float32)
+    out2 = torch.empty(n * T, C, device=tok.device, dtype=torch.bfloat16) if want_ln else None
+    stats = torch.empty(n * T, 1, 2, device=tok.device, dtype=torch.float32) if want_ln else None
+    _run(lib.ia2p_clip_embed, (ids.data_ptr(), n, T, tok.data_ptr(), V, pos.data_ptr(), pos.shape[0], C, out.data_ptr(), _ptr(out2),
+                                   _ptr(stats), _stream()), "clip_embed")
+    return (out, out2, stats) if want_ln else out
+
+
 # ------------------------------------------------------------------------------------------------ tensor-core GEMM / conv
 # split-K workspace of the tensor-core kernels: one per device (the hot path runs on ONE stream per process), registered with the
 # library before every tc launch made through this module (a thread-local pointer on the library side; re-registering is ~ns)
@@ -335,10 +361,14 @@ def _colstats_buffer(tiles, n, device):
     return torch.empty(tiles, n, 2, device=device, dtype=torch.float32) if tiles > 0 else None
 
 
+_ACT_EPI = {None: _lib.EPI_NONE, "gelu": _lib.EPI_GELU, "quick_gelu": _lib.EPI_QUICK_GELU}
+
+
 def gemm(a, w, bias=None, a2=None, rowbias=None, rows_per_batch=0, residual=None, geglu=False, out=None,
-         out_dtype=torch.bfloat16, want_ln=False, ln=None, want_colstats=False):
+         out_dtype=torch.bfloat16, want_ln=False, ln=None, want_colstats=False, act=None):
     """out = epilogue([a | a2] @ w^T).  a: [M,K1] bf16 (row-strided view allowed), w: [N,K1+K2] bf16 contiguous;
     residual bf16|fp32, out bf16|fp32 (fp32 = residual-stream tensors).
+    ``act``: None, ``"gelu"`` (exact erf) or ``"quick_gelu"`` applied after the LN correction and bias (bf16 output only).
 
     LayerNorm folding: ``want_ln=True`` (producer) returns ``(out, out_bf16, stats)`` -- a bf16 copy of the output rows and
     the per-row partial sums; ``ln=(stats, c1, eps)`` (consumer) finishes LayerNorm in the epilogue:
@@ -346,6 +376,8 @@ def gemm(a, w, bias=None, a2=None, rowbias=None, rows_per_batch=0, residual=None
     lib = _lib.load()
     _need(a, torch.bfloat16, "a", 2)
     _need(w, torch.bfloat16, "w", 2)
+    if act not in _ACT_EPI:
+        raise IA2PError(f"gemm: unsupported activation {act!r} (None, 'gelu', 'quick_gelu')")
     _ensure_tc_workspace(a.device)
     assert w.is_contiguous()
     M, K1 = a.shape
@@ -389,11 +421,11 @@ def gemm(a, w, bias=None, a2=None, rowbias=None, rows_per_batch=0, residual=None
               + (M * n_out * residual.element_size() if residual is not None else 0) + (M * N * 2 + M * 8 * 4 if want_ln else 0))
     if PROFILE is not None or TAG_ALWAYS:
         _TAG = (f"gemm M{M} N{N} K{K1 + K2}{' geglu' if geglu else ''}{' res' + str(residual.dtype)[6:] if residual is not None else ''}"
-                f" out{str(out.dtype)[6:]}{' +ln_stats' if want_ln else ''}{' ln_fold' if ln is not None else ''}")
+                f" out{str(out.dtype)[6:]}{' +ln_stats' if want_ln else ''}{' ln_fold' if ln is not None else ''}{' ' + act if act else ''}")
     _plan_step(w)
     _run(lib.ia2p_gemm_ln_bf16, (a.data_ptr(), lda, K1, _ptr(a2), lda2, K2, w.data_ptr(), out.data_ptr(), ldo, M, N,
                                   _ptr(bias), _ptr(rowbias), int(rows_per_batch), _ptr(residual), ldr, res_dt,
-                                  _DT[out.dtype], _lib.EPI_GEGLU if geglu else _lib.EPI_NONE,
+                                  _DT[out.dtype], _lib.EPI_GEGLU if geglu else _ACT_EPI[act],
                                   _ptr(out2), N, _ptr(stats), _ptr(cs), _ptr(ln_stats), ln_parts, _ptr(ln_c1), float(ln_eps),
                                   _stream()), "gemm_bf16")
     if cs is not None:
@@ -589,6 +621,23 @@ def flash_self_attn(qkv, batch, n_tokens, heads, out=None):
     _run(lib.ia2p_flash_self_attn_bf16, (qkv.data_ptr(), qkv.data_ptr() + C * es, qkv.data_ptr() + 2 * C * es, ld,
                                              out.data_ptr(), out.stride(0), batch, n_tokens, heads, 0.125, _stream()),
                "flash_self_attn")
+    return out
+
+
+def causal_self_attn(qkv, n, T, heads, out=None):
+    """Causal self-attention of n sequences of T <= 128 tokens (CLIP text towers).  qkv: [n*T, 3*C] bf16 (q | k | v);
+    returns [n*T, C] bf16."""
+    lib = _lib.load()
+    _need(qkv, torch.bfloat16, "qkv", 2)
+    C = heads * 64
+    assert qkv.shape == (n * T, 3 * C) and qkv.stride(1) == 1
+    if out is None:
+        out = torch.empty(n * T, C, device=qkv.device, dtype=torch.bfloat16)
+    es = qkv.element_size()
+    global _FLOPS
+    _FLOPS = 2.0 * n * heads * T * (T + 1) * 64               # causal half of QK^T and PV
+    _run(lib.ia2p_causal_self_attn_bf16, (qkv.data_ptr(), qkv.data_ptr() + C * es, qkv.data_ptr() + 2 * C * es, qkv.stride(0),
+                                              out.data_ptr(), out.stride(0), n, T, heads, 0.125, _stream()), "causal_self_attn")
     return out
 
 
