@@ -46,6 +46,15 @@ int ia2p_cfg_ddim_step(const void* eps2, int eps_dtype, const void* x, void* x_o
                        void* x_in_next2, int xin_dtype, int64_t batch, int64_t n,
                        float g, float c_x, float c_e, void* stream);
 
+/* ia2p_cfg_ddim_step with one guidance scale per request: sample b (rows b and batch + b of eps2) uses g[b].
+ * Replaces the same sequence as ia2p_cfg_ddim_step for a batch of requests that each carry their own `cfg`
+ * (pipeline.py:303-304 takes it per request; [3P] StableDiffusionXLPipeline applies one float to the batch).
+ * g: fp32 [batch], DEVICE memory, read when the kernel runs (a CUDA graph replays whatever it holds then).
+ * Results for sample b are bitwise those of ia2p_cfg_ddim_step with g = g[b]. */
+int ia2p_cfg_ddim_step_rows(const void* eps2, int eps_dtype, const void* x, void* x_out, int x_dtype,
+                            void* x_in_next2, int xin_dtype, int64_t batch, int64_t n,
+                            const float* g, float c_x, float c_e, void* stream);
+
 /* out = c_x*x + c_e*eps.  Replaces _backward_ddim, ddim/pnp_pipeline.py:73-85 (and DDIM step without CFG). */
 int ia2p_axpby(const void* eps, int eps_dtype, const void* x, void* x_out, int x_dtype, int64_t n,
                float c_x, float c_e, void* stream);
@@ -253,6 +262,17 @@ int ia2p_decoupled_cross_attn_bf16(const void* q, int64_t ldq,
                                    const void* k_ip, const void* v_ip, int64_t ldkv_ip, int n_ip, float ip_scale,
                                    void* out, int64_t ldo, int64_t batch, int64_t n_q, int heads,
                                    float softmax_scale, void* stream);
+
+/* ia2p_decoupled_cross_attn_bf16 with one IP scale per batch row: row b is softmax(Q Kt^T) Vt + ip_scale[b] softmax(Q Ki^T) Vi.
+ * Replaces the same attention_processor.py:371-397 sequence for a batch of requests that each set their own `scale`
+ * (ip_adapter.py:306 calls set_scale(scale) per request).  ip_scale: fp32 [batch], DEVICE memory; a CFG call has
+ * batch = 2B rows [uncond; cond] and takes cat([s, s]).  ip_scale[b] == 0 gives exactly the text-only row, and row b is
+ * bitwise the row of ia2p_decoupled_cross_attn_bf16 with the scalar ip_scale[b]. */
+int ia2p_decoupled_cross_attn_rows_bf16(const void* q, int64_t ldq,
+                                        const void* k_text, const void* v_text, int64_t ldkv, int n_text,
+                                        const void* k_ip, const void* v_ip, int64_t ldkv_ip, int n_ip, const float* ip_scale,
+                                        void* out, int64_t ldo, int64_t batch, int64_t n_q, int heads,
+                                        float softmax_scale, void* stream);
 
 /* ---------------------------------------------------------------- prior (GPT-2 trunk, weight-streaming) */
 

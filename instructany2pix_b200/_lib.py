@@ -24,6 +24,7 @@ SIGNATURES = {
     "ia2p_device_check": ([_i], _i),
     "ia2p_set_pdl": ([_i], _i),
     "ia2p_cfg_ddim_step": ([_p, _i, _p, _p, _i, _p, _i, _l, _l, _f, _f, _f, _p], _i),
+    "ia2p_cfg_ddim_step_rows": ([_p, _i, _p, _p, _i, _p, _i, _l, _l, _p, _f, _f, _p], _i),
     "ia2p_axpby": ([_p, _i, _p, _p, _i, _l, _f, _f, _p], _i),
     "ia2p_inpaint_blend": ([_p, _p, _p, _p, _p, _l, _l, _l, _f, _f, _p], _i),
     "ia2p_polar_workspace_bytes": ([], _l),
@@ -57,6 +58,7 @@ SIGNATURES = {
     "ia2p_flash_self_attn_bf16": ([_p, _p, _p, _l, _p, _l, _l, _l, _i, _f, _p], _i),
     "ia2p_causal_self_attn_bf16": ([_p, _p, _p, _l, _p, _l, _l, _l, _i, _f, _p], _i),
     "ia2p_decoupled_cross_attn_bf16": ([_p, _l, _p, _p, _l, _i, _p, _p, _l, _i, _f, _p, _l, _l, _l, _i, _f, _p], _i),
+    "ia2p_decoupled_cross_attn_rows_bf16": ([_p, _l, _p, _p, _l, _i, _p, _p, _l, _i, _p, _p, _l, _l, _l, _i, _f, _p], _i),
     "ia2p_gemm_smallm": ([_p, _l, _p, _p, _p, _l, _p, _l, _l, _l, _l, _i, _i, _p], _i),
     "ia2p_causal_attn_small_f32": ([_p, _p, _l, _l, _i, _p], _i),
     "ia2p_prior_trunk_workspace_bytes": ([_l], _l),

@@ -178,12 +178,13 @@ flash_self_attn_kernel(const __nv_bfloat16* __restrict__ q, const __nv_bfloat16*
 
 // ================================================================ decoupled cross-attention
 // All keys resident in smem: text keys padded to T1 (multiple of 16), IP keys padded to T2 (0 or 16).
+// ip_rows (nullable): per-batch-row IP scales in device memory, used instead of ip_scale.
 template <int T1, int T2>
 __global__ void __launch_bounds__(256, (T1 <= 96) ? 3 : 1)
 cross_attn_kernel(const __nv_bfloat16* __restrict__ q, long long ldq, const __nv_bfloat16* __restrict__ kt,
                   const __nv_bfloat16* __restrict__ vt, long long ldkv, int n_text, const __nv_bfloat16* __restrict__ ki,
                   const __nv_bfloat16* __restrict__ vi, long long ldkv_ip, int n_ip, float ip_scale,
-                  __nv_bfloat16* __restrict__ out, long long ldo, int n_q, float scale_log2) {
+                  const float* __restrict__ ip_rows, __nv_bfloat16* __restrict__ out, long long ldo, int n_q, float scale_log2) {
   pdl_launch_dependents();   // programmatic dependent launch: see common.cuh
   pdl_wait();
   constexpr int TK = T1 + T2;
@@ -197,6 +198,7 @@ cross_attn_kernel(const __nv_bfloat16* __restrict__ q, long long ldq, const __nv
   const int h = blockIdx.y;
   const long long b = blockIdx.z;
   const int n_qtiles = (n_q + 127) >> 7;
+  const float ips = ip_rows != nullptr ? __ldg(ip_rows + b) : ip_scale;
   // K/V of this (batch, head) are loaded ONCE per CTA; the CTA then walks its query tiles with the next Q tile in flight
   load_tile(sK, kt + b * n_text * ldkv + h * 64, ldkv, T1, n_text, tid, 256);
   load_tile(sV, vt + b * n_text * ldkv + h * 64, ldkv, T1, n_text, tid, 256);
@@ -283,7 +285,7 @@ cross_attn_kernel(const __nv_bfloat16* __restrict__ q, long long ldq, const __nv
         sum[br][r] += __shfl_xor_sync(0xffffffffu, sum[br][r], 1);
         sum[br][r] += __shfl_xor_sync(0xffffffffu, sum[br][r], 2);
         const float inv = sum[br][r] > 0.f ? 1.f / sum[br][r] : 0.f;
-        w[br][r] = br == 0 ? inv : inv * ip_scale;
+        w[br][r] = br == 0 ? inv : inv * ips;
       }
     float o[8][4];
 #pragma unroll
@@ -327,8 +329,8 @@ cross_attn_kernel(const __nv_bfloat16* __restrict__ q, long long ldq, const __nv
 
 template <int T1, int T2>
 static int launch_cross(const void* q, int64_t ldq, const void* kt, const void* vt, int64_t ldkv, int n_text, const void* ki,
-                        const void* vi, int64_t ldkv_ip, int n_ip, float ip_scale, void* out, int64_t ldo, int64_t batch,
-                        int64_t n_q, int heads, float scale, cudaStream_t st) {
+                        const void* vi, int64_t ldkv_ip, int n_ip, float ip_scale, const float* ip_rows, void* out, int64_t ldo,
+                        int64_t batch, int64_t n_q, int heads, float scale, cudaStream_t st) {
   constexpr int smem = 2 * 128 * 128 + 2 * (T1 + T2) * 128;
   IA2P_ONCE_PER_DEVICE(IA2P_CUDA(cudaFuncSetAttribute(cross_attn_kernel<T1, T2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)));
   // query tiles per (batch, head) are split over the fewest CTAs that still fill the GPU (~3 CTAs per SM): K/V loads amortise
@@ -344,7 +346,7 @@ static int launch_cross(const void* q, int64_t ldq, const void* kt, const void* 
   launch_pdl(cross_attn_kernel<T1, T2>, dim3(grid), dim3(256), smem, st, 
       static_cast<const __nv_bfloat16*>(q), ldq, static_cast<const __nv_bfloat16*>(kt), static_cast<const __nv_bfloat16*>(vt),
       ldkv, n_text, static_cast<const __nv_bfloat16*>(ki), static_cast<const __nv_bfloat16*>(vi), ldkv_ip, n_ip, ip_scale,
-      static_cast<__nv_bfloat16*>(out), ldo, (int)n_q, scale * kLog2e);
+      ip_rows, static_cast<__nv_bfloat16*>(out), ldo, (int)n_q, scale * kLog2e);
   IA2P_LAUNCH_CHECK();
   return 0;
 }
@@ -480,8 +482,8 @@ namespace ia2p {
 int launch_fa_tc(const void* q, const void* k, const void* v, int64_t ld, void* out, int64_t ldo, int64_t batch,
                  int64_t n_tokens, int heads, float softmax_scale, cudaStream_t st);
 int launch_xattn_tc(const void* q, int64_t ldq, const void* kt, const void* vt, int64_t ldkv, int n_text, const void* ki,
-                    const void* vi, int64_t ldkv_ip, int n_ip, float ip_scale, void* out, int64_t ldo, int64_t batch, int64_t n_q,
-                    int heads, float scale, cudaStream_t st, bool* handled);
+                    const void* vi, int64_t ldkv_ip, int n_ip, float ip_scale, const float* ip_rows, void* out, int64_t ldo,
+                    int64_t batch, int64_t n_q, int heads, float scale, cudaStream_t st, bool* handled);
 }
 using namespace ia2p;
 
@@ -528,10 +530,10 @@ extern "C" int ia2p_causal_self_attn_bf16(const void* q, const void* k, const vo
   return launch_causal<128>(q, k, v, ld, out, ldo, n, T, heads, softmax_scale, st);
 }
 
-extern "C" int ia2p_decoupled_cross_attn_bf16(const void* q, int64_t ldq, const void* k_text, const void* v_text, int64_t ldkv,
-                                              int n_text, const void* k_ip, const void* v_ip, int64_t ldkv_ip, int n_ip,
-                                              float ip_scale, void* out, int64_t ldo, int64_t batch, int64_t n_q, int heads,
-                                              float softmax_scale, void* stream) {
+// ip_rows == nullptr: one IP scale for the batch (ia2p_decoupled_cross_attn_bf16); else ip_rows[batch] on the device
+static int cross_attn_launch(const void* q, int64_t ldq, const void* k_text, const void* v_text, int64_t ldkv, int n_text,
+                             const void* k_ip, const void* v_ip, int64_t ldkv_ip, int n_ip, float ip_scale, const float* ip_rows,
+                             void* out, int64_t ldo, int64_t batch, int64_t n_q, int heads, float softmax_scale, void* stream) {
   if (int e = check_device()) return e;
   IA2P_REQUIRE(q && k_text && v_text && out && batch > 0 && n_q > 0 && heads > 0, IA2P_E_ARG, "cross_attn: bad arguments");
   IA2P_REQUIRE(n_text > 0 && n_text <= 128 && n_ip >= 0 && n_ip <= 16, IA2P_E_SHAPE, "cross_attn: n_text=%d (<=128) n_ip=%d (<=16)", n_text, n_ip);
@@ -541,13 +543,14 @@ extern "C" int ia2p_decoupled_cross_attn_bf16(const void* q, int64_t ldq, const 
   static const bool legacy_cross = [] { const char* e = getenv("IA2P_XATTN_IMPL"); return e != nullptr && e[0] == 'm'; }();   // A/B only
   if (!use_legacy_attn() && !legacy_cross) {                  // tcgen05 kernel (xattn_tc.cu) whenever all keys fit 128 columns
     bool handled = false;
-    const int e = launch_xattn_tc(q, ldq, k_text, v_text, ldkv, n_text, k_ip, v_ip, ldkv_ip, n_ip, ip_scale, out, ldo, batch, n_q, heads,
-                                  softmax_scale, st, &handled);
+    const int e = launch_xattn_tc(q, ldq, k_text, v_text, ldkv, n_text, k_ip, v_ip, ldkv_ip, n_ip, ip_scale, ip_rows, out, ldo, batch,
+                                  n_q, heads, softmax_scale, st, &handled);
     if (e != 0 || handled) return e;
   }
   const int t1 = n_text <= 80 ? 80 : (n_text <= 96 ? 96 : 128);
 #define IA2P_CROSS(T1_, T2_) \
-  return launch_cross<T1_, T2_>(q, ldq, k_text, v_text, ldkv, n_text, k_ip, v_ip, ldkv_ip, n_ip, ip_scale, out, ldo, batch, n_q, heads, softmax_scale, st)
+  return launch_cross<T1_, T2_>(q, ldq, k_text, v_text, ldkv, n_text, k_ip, v_ip, ldkv_ip, n_ip, ip_scale, ip_rows, out, ldo, batch, n_q, \
+                                heads, softmax_scale, st)
   if (n_ip > 0) {
     if (t1 == 80) IA2P_CROSS(80, 16);
     if (t1 == 96) IA2P_CROSS(96, 16);
@@ -558,4 +561,22 @@ extern "C" int ia2p_decoupled_cross_attn_bf16(const void* q, int64_t ldq, const 
     IA2P_CROSS(128, 0);
   }
 #undef IA2P_CROSS
+}
+
+extern "C" int ia2p_decoupled_cross_attn_bf16(const void* q, int64_t ldq, const void* k_text, const void* v_text, int64_t ldkv,
+                                              int n_text, const void* k_ip, const void* v_ip, int64_t ldkv_ip, int n_ip,
+                                              float ip_scale, void* out, int64_t ldo, int64_t batch, int64_t n_q, int heads,
+                                              float softmax_scale, void* stream) {
+  return cross_attn_launch(q, ldq, k_text, v_text, ldkv, n_text, k_ip, v_ip, ldkv_ip, n_ip, ip_scale, nullptr, out, ldo, batch, n_q,
+                           heads, softmax_scale, stream);
+}
+
+extern "C" int ia2p_decoupled_cross_attn_rows_bf16(const void* q, int64_t ldq, const void* k_text, const void* v_text,
+                                                   int64_t ldkv, int n_text, const void* k_ip, const void* v_ip, int64_t ldkv_ip,
+                                                   int n_ip, const float* ip_scale, void* out, int64_t ldo, int64_t batch,
+                                                   int64_t n_q, int heads, float softmax_scale, void* stream) {
+  IA2P_REQUIRE(ip_scale != nullptr, IA2P_E_ARG, "cross_attn_rows: null IP-scale array");
+  IA2P_REQUIRE((reinterpret_cast<uintptr_t>(ip_scale) & 3) == 0, IA2P_E_ALIGN, "cross_attn_rows: ip_scale must be 4-byte aligned");
+  return cross_attn_launch(q, ldq, k_text, v_text, ldkv, n_text, k_ip, v_ip, ldkv_ip, n_ip, 0.f, ip_scale, out, ldo, batch, n_q,
+                           heads, softmax_scale, stream);
 }

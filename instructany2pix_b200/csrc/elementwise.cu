@@ -45,13 +45,17 @@ template <> __device__ __forceinline__ void store8<__half>(__half* p, const floa
 // ---------------------------------------------------------------- CFG + DDIM (one pass over the latents)
 // VEC = true: 8 elements per thread and iteration through 128-bit loads / stores; VEC = false: scalar fallback for unaligned or
 // ragged sizes.  total = batch * n; eps_u at [i], eps_c at [total + i].
-template <typename TE, typename TX, typename TI, bool VEC>
+// ROWS = true: the guidance scale of sample i / n is g_rows[i / n] (one request per batch row); the VEC variant needs n % 8 == 0,
+// so the eight elements of a thread belong to one sample and one load serves them.  ROWS = false compiles to the scalar-g kernel.
+template <typename TE, typename TX, typename TI, bool VEC, bool ROWS>
 __global__ void cfg_ddim_kernel(const TE* __restrict__ eps2, const TX* __restrict__ x, TX* __restrict__ x_out,
-                                TI* __restrict__ x_in2, long long total, float g, float cx, float ce) {
+                                TI* __restrict__ x_in2, long long total, float g_scalar, float cx, float ce,
+                                const float* __restrict__ g_rows, long long n) {
   pdl_launch_dependents();   // programmatic dependent launch: see common.cuh
   pdl_wait();
   constexpr int W = VEC ? 8 : 1;
   for (long long i = (blockIdx.x * (long long)blockDim.x + threadIdx.x) * W; i < total; i += (long long)gridDim.x * blockDim.x * W) {
+    const float g = ROWS ? __ldg(g_rows + i / n) : g_scalar;
     if constexpr (VEC) {
       float eu[8], ec[8], xv[8], v[8];
       load8(eps2 + i, eu);
@@ -489,9 +493,10 @@ using namespace ia2p;
     default: set_error("unknown dtype code %d", (int)(code)); return IA2P_E_ARG; \
   }
 
-extern "C" int ia2p_cfg_ddim_step(const void* eps2, int eps_dtype, const void* x, void* x_out, int x_dtype,
-                                  void* x_in_next2, int xin_dtype, int64_t batch, int64_t n, float g, float c_x,
-                                  float c_e, void* stream) {
+// g_rows == nullptr: one guidance scale `g` for the batch (ia2p_cfg_ddim_step); else g_rows[batch] on the device
+static int cfg_ddim_launch(const void* eps2, int eps_dtype, const void* x, void* x_out, int x_dtype, void* x_in_next2,
+                           int xin_dtype, int64_t batch, int64_t n, float g, const float* g_rows, float c_x, float c_e,
+                           void* stream) {
   if (int e = check_device()) return e;
   IA2P_REQUIRE(eps2 && x && x_out && batch > 0 && n > 0, IA2P_E_ARG, "cfg_ddim_step: null pointer or empty shape");
   const long long total = batch * n;
@@ -499,21 +504,38 @@ extern "C" int ia2p_cfg_ddim_step(const void* eps2, int eps_dtype, const void* x
   if (x_in_next2 == nullptr) xin_dtype = x_dtype;
   auto esz = [](int dt) { return dt == IA2P_F32 ? 4ll : 2ll; };
   auto al16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
-  // 128-bit path: every 8-element group of every array starts on a 16-byte boundary (the second halves start at `total`)
+  // 128-bit path: every 8-element group of every array starts on a 16-byte boundary (the second halves start at `total`); with
+  // per-row scales a group must also lie inside one sample
   const bool vec = total % 8 == 0 && al16(eps2) && al16(x) && al16(x_out) && (x_in_next2 == nullptr || al16(x_in_next2)) &&
-                   (total * esz(eps_dtype)) % 16 == 0 && (total * esz(xin_dtype)) % 16 == 0;
+                   (total * esz(eps_dtype)) % 16 == 0 && (total * esz(xin_dtype)) % 16 == 0 && (g_rows == nullptr || n % 8 == 0);
   const int grid = grid_for(vec ? total / 8 : total, 256);
-  if (vec) {
-    DISPATCH_DTYPE(eps_dtype, TE, DISPATCH_DTYPE(x_dtype, TX, DISPATCH_DTYPE(xin_dtype, TI,
-        (launch_pdl(cfg_ddim_kernel<TE, TX, TI, true>, dim3(grid), dim3(256), 0, st, static_cast<const TE*>(eps2), static_cast<const TX*>(x),
-                    static_cast<TX*>(x_out), static_cast<TI*>(x_in_next2), total, g, c_x, c_e)))));
+#define IA2P_CFG_DDIM(VEC_, ROWS_)                                                                                              \
+  DISPATCH_DTYPE(eps_dtype, TE, DISPATCH_DTYPE(x_dtype, TX, DISPATCH_DTYPE(xin_dtype, TI,                                       \
+      (launch_pdl(cfg_ddim_kernel<TE, TX, TI, VEC_, ROWS_>, dim3(grid), dim3(256), 0, st, static_cast<const TE*>(eps2),         \
+                  static_cast<const TX*>(x), static_cast<TX*>(x_out), static_cast<TI*>(x_in_next2), total, g, c_x, c_e, g_rows, \
+                  (long long)n)))))
+  if (g_rows == nullptr) {
+    if (vec) { IA2P_CFG_DDIM(true, false); } else { IA2P_CFG_DDIM(false, false); }
   } else {
-    DISPATCH_DTYPE(eps_dtype, TE, DISPATCH_DTYPE(x_dtype, TX, DISPATCH_DTYPE(xin_dtype, TI,
-        (launch_pdl(cfg_ddim_kernel<TE, TX, TI, false>, dim3(grid), dim3(256), 0, st, static_cast<const TE*>(eps2), static_cast<const TX*>(x),
-                    static_cast<TX*>(x_out), static_cast<TI*>(x_in_next2), total, g, c_x, c_e)))));
+    if (vec) { IA2P_CFG_DDIM(true, true); } else { IA2P_CFG_DDIM(false, true); }
   }
+#undef IA2P_CFG_DDIM
   IA2P_LAUNCH_CHECK();
   return 0;
+}
+
+extern "C" int ia2p_cfg_ddim_step(const void* eps2, int eps_dtype, const void* x, void* x_out, int x_dtype,
+                                  void* x_in_next2, int xin_dtype, int64_t batch, int64_t n, float g, float c_x,
+                                  float c_e, void* stream) {
+  return cfg_ddim_launch(eps2, eps_dtype, x, x_out, x_dtype, x_in_next2, xin_dtype, batch, n, g, nullptr, c_x, c_e, stream);
+}
+
+extern "C" int ia2p_cfg_ddim_step_rows(const void* eps2, int eps_dtype, const void* x, void* x_out, int x_dtype,
+                                       void* x_in_next2, int xin_dtype, int64_t batch, int64_t n, const float* g,
+                                       float c_x, float c_e, void* stream) {
+  IA2P_REQUIRE(g != nullptr, IA2P_E_ARG, "cfg_ddim_step_rows: null guidance-scale array");
+  IA2P_REQUIRE((reinterpret_cast<uintptr_t>(g) & 3) == 0, IA2P_E_ALIGN, "cfg_ddim_step_rows: g must be 4-byte aligned");
+  return cfg_ddim_launch(eps2, eps_dtype, x, x_out, x_dtype, x_in_next2, xin_dtype, batch, n, 0.f, g, c_x, c_e, stream);
 }
 
 extern "C" int ia2p_axpby(const void* eps, int eps_dtype, const void* x, void* x_out, int x_dtype, int64_t n, float c_x,

@@ -31,15 +31,17 @@ struct alignas(64) XaMaps {
 
 constexpr int kXaQ = 128 * 128;    // bytes of a Q tile: 128 rows x 64 bf16
 
-template <int T1, int T2>
+// ROWS = true: batch row b weighs its IP branch by ip_rows[b] (one request per row) instead of ip_scale
+template <int T1, int T2, bool ROWS>
 __global__ void __launch_bounds__(192, 2)
 xattn_tc_kernel(const __grid_constant__ XaMaps maps, int n_q, int n_text, int n_ip,
-                int heads, int n_items, float ip_scale, float scale_log2) {
+                int heads, int n_items, float ip_scale, float scale_log2, const float* __restrict__ ip_rows) {
   constexpr int TK = T1 + T2;
   constexpr int KV = TK * 128;                          // bytes of the K (or V) rows of one head
   constexpr int STAGE = kXaQ + 2 * KV;
   constexpr int NCH = (TK + 31) / 32;                   // 32-column chunks of S
   static_assert(T1 % 16 == 0 && (T2 == 0 || T2 == 16) && TK <= 128, "key padding");
+  static_assert(!ROWS || T2 > 0, "per-row IP scales need IP keys");
   pdl_launch_dependents();
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw = smem_u32(smem_raw);
@@ -179,7 +181,8 @@ xattn_tc_kernel(const __grid_constant__ XaMaps maps, int n_q, int n_text, int n_
         }
       }
       if (T2 > 0) {
-        const float f = (li > 0.f) ? ip_scale * lt / li : 0.f;
+        const float s = ROWS ? __ldg(ip_rows + b) : ip_scale;
+        const float f = (li > 0.f) ? s * lt / li : 0.f;
 #pragma unroll
         for (int i = 0; i < T2; i += 2) pk[(T1 + i) >> 1] = pack_bf16x2(pip[i] * f, pip[i + 1] * f);
       }
@@ -234,10 +237,10 @@ xattn_tc_kernel(const __grid_constant__ XaMaps maps, int n_q, int n_text, int n_
   }
 }
 
-template <int T1, int T2>
+template <int T1, int T2, bool ROWS>
 static int launch_xa(const void* q, int64_t ldq, const void* kt, const void* vt, int64_t ldkv, int n_text, const void* ki,
-                     const void* vi, int64_t ldkv_ip, int n_ip, float ip_scale, void* out, int64_t ldo, int64_t batch, int64_t n_q,
-                     int heads, float scale, cudaStream_t st) {
+                     const void* vi, int64_t ldkv_ip, int n_ip, float ip_scale, const float* ip_rows, void* out, int64_t ldo,
+                     int64_t batch, int64_t n_q, int heads, float scale, cudaStream_t st) {
   constexpr int TK = T1 + T2;
   constexpr int smem = 2 * (kXaQ + 2 * TK * 128) + kXaQ + 1024 + 128;
   XaMaps maps;
@@ -252,35 +255,41 @@ static int launch_xa(const void* q, int64_t ldq, const void* kt, const void* vt,
     if (int e = make_map_3d_bf16(&maps.vi, vi, heads * 64, ldkv_ip, n_ip, batch, T2, "cross_attn")) return e;
   }
   IA2P_ONCE_PER_DEVICE(
-      IA2P_CUDA(cudaFuncSetAttribute(xattn_tc_kernel<T1, T2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-      IA2P_CUDA(cudaFuncSetAttribute(xattn_tc_kernel<T1, T2>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)));
+      IA2P_CUDA(cudaFuncSetAttribute(xattn_tc_kernel<T1, T2, ROWS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+      IA2P_CUDA(cudaFuncSetAttribute(xattn_tc_kernel<T1, T2, ROWS>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)));
   const long long n_items = (long long)((n_q + 127) / 128) * heads * batch;
   IA2P_REQUIRE(n_items < (1ll << 31), IA2P_E_SHAPE, "cross_attn: too many work items");
   const long long resident = 2LL * sm_count();
   const dim3 grid((unsigned)(n_items < resident ? n_items : resident));
-  launch_pdl(xattn_tc_kernel<T1, T2>, dim3(grid), dim3(192), smem, st, maps, (int)n_q, n_text, n_ip, heads, (int)n_items, ip_scale,
-             scale * 1.4426950408889634f);
+  launch_pdl(xattn_tc_kernel<T1, T2, ROWS>, dim3(grid), dim3(192), smem, st, maps, (int)n_q, n_text, n_ip, heads, (int)n_items,
+             ip_scale, scale * 1.4426950408889634f, ip_rows);
   IA2P_LAUNCH_CHECK();
   return 0;
 }
 
-// -> 0 launched | < 0 / > 0 error | IA2P_XA_UNSUPPORTED: shape outside this kernel (caller falls back to the mma.sync kernel)
+// -> 0 launched | < 0 / > 0 error; *handled = false: shape outside this kernel (caller falls back to the mma.sync kernel).
+// ip_rows (nullable, used only when n_ip > 0): per-batch-row IP scales in device memory instead of ip_scale.
 int launch_xattn_tc(const void* q, int64_t ldq, const void* kt, const void* vt, int64_t ldkv, int n_text, const void* ki,
-                    const void* vi, int64_t ldkv_ip, int n_ip, float ip_scale, void* out, int64_t ldo, int64_t batch, int64_t n_q,
-                    int heads, float scale, cudaStream_t st, bool* handled) {
+                    const void* vi, int64_t ldkv_ip, int n_ip, float ip_scale, const float* ip_rows, void* out, int64_t ldo,
+                    int64_t batch, int64_t n_q, int heads, float scale, cudaStream_t st, bool* handled) {
   *handled = true;
   const int t1 = n_text <= 80 ? 80 : (n_text <= 96 ? 96 : (n_text <= 112 ? 112 : 128));
-#define IA2P_XA(T1_, T2_) \
-  return launch_xa<T1_, T2_>(q, ldq, kt, vt, ldkv, n_text, ki, vi, ldkv_ip, n_ip, ip_scale, out, ldo, batch, n_q, heads, scale, st)
-  if (n_ip > 0) {
-    if (t1 == 80) IA2P_XA(80, 16);
-    if (t1 == 96) IA2P_XA(96, 16);
-    if (t1 == 112) IA2P_XA(112, 16);
+#define IA2P_XA(T1_, T2_, ROWS_) \
+  return launch_xa<T1_, T2_, ROWS_>(q, ldq, kt, vt, ldkv, n_text, ki, vi, ldkv_ip, n_ip, ip_scale, ip_rows, out, ldo, batch, n_q, heads, \
+                                    scale, st)
+  if (n_ip > 0 && ip_rows != nullptr) {
+    if (t1 == 80) IA2P_XA(80, 16, true);
+    if (t1 == 96) IA2P_XA(96, 16, true);
+    if (t1 == 112) IA2P_XA(112, 16, true);
+  } else if (n_ip > 0) {
+    if (t1 == 80) IA2P_XA(80, 16, false);
+    if (t1 == 96) IA2P_XA(96, 16, false);
+    if (t1 == 112) IA2P_XA(112, 16, false);
   } else {
-    if (t1 == 80) IA2P_XA(80, 0);
-    if (t1 == 96) IA2P_XA(96, 0);
-    if (t1 == 112) IA2P_XA(112, 0);
-    IA2P_XA(128, 0);
+    if (t1 == 80) IA2P_XA(80, 0, false);
+    if (t1 == 96) IA2P_XA(96, 0, false);
+    if (t1 == 112) IA2P_XA(112, 0, false);
+    IA2P_XA(128, 0, false);
   }
 #undef IA2P_XA
   *handled = false;                       // 112 < n_text <= 128 together with IP keys: more than 128 key columns

@@ -143,9 +143,20 @@ def _f32(t, name):
     return None if t is None else _need(t, torch.float32, name).contiguous()
 
 
+def _row_scales(t, batch, name):
+    """a per-request scale vector: contiguous fp32 [batch] on the CUDA device (its values are read when the kernel runs)"""
+    _need(t, torch.float32, name, 1)
+    if t.shape[0] != batch:
+        raise ValueError(f"{name}: {t.shape[0]} values for a batch of {batch} rows")
+    if not t.is_contiguous():
+        raise IA2PError(f"{name}: expected a contiguous tensor")
+    return t
+
+
 # ------------------------------------------------------------------------------------------------ sampler epilogues
 def cfg_ddim_step(eps2, x, g, c_x, c_e, x_out=None, x_in_next2=None):
-    """x_out = c_x*x + c_e*(eps_u + g*(eps_c - eps_u)); eps2 = [uncond; cond] (custom_pipelines.py:348-357)."""
+    """x_out = c_x*x + c_e*(eps_u + g*(eps_c - eps_u)); eps2 = [uncond; cond] (custom_pipelines.py:348-357).
+    ``g``: a float for the whole batch, or a contiguous fp32 CUDA tensor [batch] with one guidance scale per request."""
     lib = _lib.load()
     eps2, x = eps2.contiguous(), x.contiguous()
     batch = x.shape[0]
@@ -153,8 +164,13 @@ def cfg_ddim_step(eps2, x, g, c_x, c_e, x_out=None, x_in_next2=None):
     assert eps2.numel() == 2 * x.numel()
     if x_out is None:
         x_out = torch.empty_like(x)
-    _run(lib.ia2p_cfg_ddim_step, (eps2.data_ptr(), _DT[eps2.dtype], x.data_ptr(), x_out.data_ptr(), _DT[x.dtype],
-                                      _ptr(x_in_next2), _DT[x_in_next2.dtype] if x_in_next2 is not None else F32,
+    xin = (_ptr(x_in_next2), _DT[x_in_next2.dtype] if x_in_next2 is not None else F32)
+    if isinstance(g, torch.Tensor):
+        g = _row_scales(g, batch, "cfg_ddim_step: g")
+        _run(lib.ia2p_cfg_ddim_step_rows, (eps2.data_ptr(), _DT[eps2.dtype], x.data_ptr(), x_out.data_ptr(), _DT[x.dtype], *xin,
+                                           batch, n, g.data_ptr(), float(c_x), float(c_e), _stream()), "cfg_ddim_step_rows")
+        return x_out
+    _run(lib.ia2p_cfg_ddim_step, (eps2.data_ptr(), _DT[eps2.dtype], x.data_ptr(), x_out.data_ptr(), _DT[x.dtype], *xin,
                                       batch, n, float(g), float(c_x), float(c_e), _stream()), "cfg_ddim_step")
     return x_out
 
@@ -642,7 +658,8 @@ def causal_self_attn(qkv, n, T, heads, out=None):
 
 
 def cross_attn(q, kv_text, n_text, kv_ip, n_ip, ip_scale, batch, n_q, heads, out=None):
-    """Decoupled cross-attention.  q: [batch*n_q, C]; kv_text: [batch*n_text, 2C] (k | v); kv_ip: [batch*n_ip, 2C] | None."""
+    """Decoupled cross-attention.  q: [batch*n_q, C]; kv_text: [batch*n_text, 2C] (k | v); kv_ip: [batch*n_ip, 2C] | None.
+    ``ip_scale``: a float for the whole batch, or a contiguous fp32 CUDA tensor [batch] with one IP scale per row."""
     lib = _lib.load()
     _need(q, torch.bfloat16, "q", 2)
     _need(kv_text, torch.bfloat16, "kv_text", 2)
@@ -659,10 +676,13 @@ def cross_attn(q, kv_text, n_text, kv_ip, n_ip, ip_scale, batch, n_q, heads, out
         out = torch.empty(batch * n_q, C, device=q.device, dtype=torch.bfloat16)
     global _FLOPS
     _FLOPS = 4.0 * batch * heads * n_q * (n_text + n_ip) * 64
-    _run(lib.ia2p_decoupled_cross_attn_bf16, (q.data_ptr(), q.stride(0), kv_text.data_ptr(), kv_text.data_ptr() + C * es,
-                                                  kv_text.stride(0), n_text, kip, vip, ldip, n_ip, float(ip_scale),
-                                                  out.data_ptr(), out.stride(0), batch, n_q, heads, 0.125, _stream()),
-               "decoupled_cross_attn")
+    if isinstance(ip_scale, torch.Tensor):
+        fn, scale, what = lib.ia2p_decoupled_cross_attn_rows_bf16, _row_scales(ip_scale, batch, "cross_attn: ip_scale").data_ptr(), \
+            "decoupled_cross_attn_rows"
+    else:
+        fn, scale, what = lib.ia2p_decoupled_cross_attn_bf16, float(ip_scale), "decoupled_cross_attn"
+    _run(fn, (q.data_ptr(), q.stride(0), kv_text.data_ptr(), kv_text.data_ptr() + C * es, kv_text.stride(0), n_text, kip, vip, ldip,
+              n_ip, scale, out.data_ptr(), out.stride(0), batch, n_q, heads, 0.125, _stream()), what)
     return out
 
 

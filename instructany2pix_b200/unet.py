@@ -526,28 +526,29 @@ class B200UNet(nn.Module):
             return SimpleNamespace(sample=eps)
         return (eps,)
 
-    def forward_core(self, sample, rowbias, kv, batch, out_dtype=torch.float32):
+    def forward_core(self, sample, rowbias, kv, batch, out_dtype=torch.float32, ip_scales=None):
         """All per-step device work (capturable in a CUDA graph: no host sync, no data-dependent control flow).
-        ``sample`` may hold ``batch`` or ``batch // 2`` images (CFG duplication is folded into conv_in)."""
+        ``sample`` may hold ``batch`` or ``batch // 2`` images (CFG duplication is folded into conv_in).
+        ``ip_scales``: optional fp32 CUDA tensor [batch], the IP scale of every UNet row (a CFG batch takes cat([s, s])); every
+        cross-attention reads it instead of the processors' ``scale``, at run time (a captured graph replays its current values)."""
         P = self.prepare()
         cfg = self.config
         G = cfg.norm_num_groups
         kv_t, kv_i, n_text, n_ip = kv
-        _, ip_scale = self._ip_state()
         # weight prefetch plan: keyed by everything that fixes the launch order (packed weights, batch, resolution, processors)
         pkey = (id(P), batch, tuple(sample.shape[-2:]), n_text, n_ip, self._proc_version)
         plan = self._wplans.setdefault(pkey, {"seq": [], "ready": False})
         ops.plan_begin(plan)
         try:
-            return self._forward_core(sample, rowbias, kv, batch, out_dtype, P)
+            return self._forward_core(sample, rowbias, kv, batch, out_dtype, P, ip_scales)
         finally:
             ops.plan_end()
 
-    def _forward_core(self, sample, rowbias, kv, batch, out_dtype, P):
+    def _forward_core(self, sample, rowbias, kv, batch, out_dtype, P, ip_scales=None):
         cfg = self.config
         G = cfg.norm_num_groups
         kv_t, kv_i, n_text, n_ip = kv
-        _, ip_scale = self._ip_state()
+        ip_scale = self._ip_state()[1] if ip_scales is None else ip_scales
 
         SD = self.stream_dtype
 

@@ -21,6 +21,7 @@ import torch.nn as nn
 
 from . import ops
 from .packing import pack_conv3x3, pack_conv3x3_up2x, pack_conv_out
+from .sampler import randn_per_request
 
 
 @dataclass
@@ -250,7 +251,7 @@ class B200VAE(nn.Module):
     @torch.no_grad()
     def encode(self, images, noise=None, generator=None, sample=True, scaled=True):
         """images (B,3,H,W) in [-1, 1] -> latents (B,4,H/8,W/8) fp32 = ``latent_dist.sample() * scaling_factor``
-        (``sample=False``: the mode).  ``noise`` may be supplied for parity tests."""
+        (``sample=False``: the mode).  ``noise`` may be supplied for parity tests; ``generator`` may be one generator per image."""
         P, cfg = self.prepare(), self.config
         G = cfg.norm_num_groups
         x = ops.conv_in(images.to(self.device, torch.float32), *P["encoder.conv_in"], out_dtype=torch.float32)
@@ -270,5 +271,5 @@ class B200VAE(nn.Module):
         # DiagonalGaussianDistribution.sample ([3P]): mean + exp(0.5 * clamp(logvar, -30, 20)) * noise
         if noise is None:
             B, C2, h, w = moments.shape
-            noise = torch.randn((B, C2 // 2, h, w), device=moments.device, dtype=torch.float32, generator=generator)
+            noise = randn_per_request((B, C2 // 2, h, w), moments.device, generator)
         return ops.gaussian_sample(moments, noise.to(moments.device, torch.float32), sf)
