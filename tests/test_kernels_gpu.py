@@ -1,4 +1,5 @@
-"""GPU unit tests of every C-ABI kernel against a plain torch fp32 reference of the same op (tolerances stated inline)."""
+"""GPU unit tests of every C-ABI kernel against a plain torch fp32 reference of the same op (tolerances stated inline).
+Every test runs on poisoned allocations (tests/_poison.py), so each one also proves that its kernels write their whole output."""
 import math
 
 import pytest
@@ -8,6 +9,13 @@ import torch.nn.functional as F
 pytestmark = pytest.mark.gpu
 
 from instructany2pix_b200 import ops  # noqa: E402
+from tests._poison import poisoned  # noqa: E402
+
+
+@pytest.fixture(autouse=True)
+def _poisoned_allocations():
+    with poisoned():
+        yield
 
 DEV = "cuda"
 # references must be true fp32 (cuDNN/cuBLAS default to TF32 for fp32 inputs)
@@ -505,6 +513,39 @@ def test_upsample_conv_in_out():
     wo, bo = rnd(4, 64, 3, 3, dtype=torch.float32, scale=0.05), rnd(4, dtype=torch.float32)
     z = ops.conv_out(h, wo.permute(0, 2, 3, 1).contiguous(), bo)
     assert rel(z, F.conv2d(h.float().permute(0, 3, 1, 2), wo, bo, padding=1)) < 1e-4
+
+
+@pytest.mark.parametrize("noise", [False, True])
+@pytest.mark.parametrize("B", [1, 3])
+def test_inpaint_blend(B, noise):
+    """out = (1 - mask) (c_x orig + c_e noise) + mask latents, one mask per image broadcast over the channels"""
+    lat, orig = rnd(B, 4, 40, 24, dtype=torch.float32, seed=1), rnd(B, 4, 40, 24, dtype=torch.float32, seed=2)
+    nz = rnd(B, 4, 40, 24, dtype=torch.float32, seed=3) if noise else None
+    mask = torch.rand(B, 1, 40, 24, generator=torch.Generator().manual_seed(4)).round().to(DEV)
+    mask[:, :, :3] = 0.25                                     # soft-edged rows as well as hard 0 / 1
+    out = ops.inpaint_blend(lat, orig, nz, mask, 0.8, 0.6)
+    keep = 0.8 * orig.double() + (0.6 * nz.double() if noise else 0)
+    ref = (1 - mask.double()) * keep + mask.double() * lat.double()
+    assert ((out.double() - ref).abs() <= 1e-6 * (keep.abs() + lat.double().abs()) + 1e-7).all()
+    if B > 1:                                                  # each image blends with its own mask
+        assert not torch.equal(mask[0], mask[1])
+
+
+@pytest.mark.parametrize("C", [3, 4, 8])
+def test_conv_out_tc(C):
+    """conv_out on the tensor cores: 3x3 conv with the C output channels zero-padded to 32, then the NHWC-prefix -> NCHW copy"""
+    from instructany2pix_b200.packing import pack_conv_out
+    B, H, W, Cin = 2, 24, 40, 128
+    x = rnd(B, H, W, Cin)
+    w, b = rnd(C, Cin, 3, 3, scale=(9 * Cin) ** -0.5, dtype=torch.float32), rnd(C, dtype=torch.float32)
+    w32, b32 = pack_conv_out(w, b)
+    out = ops.conv_out_tc(x, w32, b32, C)
+    assert out.shape == (B, C, H, W) and out.dtype == torch.float32
+    wq = w32[:C].reshape(C, 3, 3, Cin).permute(0, 3, 1, 2).double()          # the bf16 weights the kernel multiplies by
+    xn = x.double().permute(0, 3, 1, 2)
+    ref = F.conv2d(xn, wq, b.double(), padding=1)
+    mag = F.conv2d(xn.abs(), wq.abs(), b.double().abs(), padding=1)
+    assert ((out.double() - ref).abs() <= 9 * Cin * 2.0 ** -23 * mag + 1e-6).all()
 
 
 @pytest.mark.parametrize("M,N,K,act_in,act", [(22, 3072, 1024, 0, 0), (28, 1024, 4096, 0, 1), (2, 1280, 320, 2, 0),
