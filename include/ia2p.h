@@ -55,6 +55,25 @@ int ia2p_cfg_ddim_step_rows(const void* eps2, int eps_dtype, const void* x, void
                             void* x_in_next2, int xin_dtype, int64_t batch, int64_t n,
                             const float* g, float c_x, float c_e, void* stream);
 
+/* CFG combine + linear scheduler update with every coefficient per row (continuous batching: each batch row is a slot at its own
+ * position in its own schedule).  g, c_x, c_e: fp32 [batch], DEVICE memory, read when the kernel runs.  Row b of x_out is bitwise
+ * ia2p_cfg_ddim_step with the scalars (g[b], c_x[b], c_e[b]); g = 0, c_x = 1, c_e = 0 leaves a finite row unchanged.
+ * x_in_next (nullable, with s_in fp32 [batch] on the device): [batch, n] receives s_in[b] * x_out, the row's next UNet input
+ * (Euler's x / sqrt(sigma_next^2 + 1)), bitwise ia2p_axpby(x_out, x_out, s_in[b], 0) for finite values.  NOT duplicated. */
+int ia2p_cfg_step_coef_rows(const void* eps2, int eps_dtype, const void* x, void* x_out, int x_dtype,
+                            void* x_in_next, int xin_dtype, int64_t batch, int64_t n,
+                            const float* g, const float* c_x, const float* c_e, const float* s_in, void* stream);
+
+/* The step's blocked time-embedding rowbias of an S-slot CFG batch, gathered from per-slot tables, then every slot's step counter
+ * advanced (a second, one-block launch).  tables: fp32 [slots, rows, 2 * sumC], row k of slot s = what
+ * time_rowbias_table(timesteps, pair, 2) gives for the slot's request at step k; coef_tables: fp32 [slots, rows, ncoef];
+ * step: int32 [slots], the row each slot reads, +1 after the gather up to rows - 1 (the sentinel row an idle slot stays on).
+ * rowbias: fp32 [2 * slots * sumC], blocked per ResnetBlock r as [2 * slots, C_r] (slot s owns rows s and slots + s);
+ * coef: fp32 [ncoef, slots].  block_lo: HOST array [nblocks + 1] of the blocks' column offsets (0 = first, last = sumC);
+ * nblocks <= 64.  All device arrays are read when the kernels run. */
+int ia2p_rowbias_gather(const float* tables, const float* coef_tables, int* step, float* rowbias, float* coef,
+                        int64_t slots, int64_t rows, const int64_t* block_lo, int64_t nblocks, int64_t ncoef, void* stream);
+
 /* out = c_x*x + c_e*eps.  Replaces _backward_ddim, ddim/pnp_pipeline.py:73-85 (and DDIM step without CFG). */
 int ia2p_axpby(const void* eps, int eps_dtype, const void* x, void* x_out, int x_dtype, int64_t n,
                float c_x, float c_e, void* stream);

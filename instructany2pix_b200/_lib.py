@@ -25,6 +25,8 @@ SIGNATURES = {
     "ia2p_set_pdl": ([_i], _i),
     "ia2p_cfg_ddim_step": ([_p, _i, _p, _p, _i, _p, _i, _l, _l, _f, _f, _f, _p], _i),
     "ia2p_cfg_ddim_step_rows": ([_p, _i, _p, _p, _i, _p, _i, _l, _l, _p, _f, _f, _p], _i),
+    "ia2p_cfg_step_coef_rows": ([_p, _i, _p, _p, _i, _p, _i, _l, _l, _p, _p, _p, _p, _p], _i),
+    "ia2p_rowbias_gather": ([_p, _p, _p, _p, _p, _l, _l, _p, _l, _l, _p], _i),
     "ia2p_axpby": ([_p, _i, _p, _p, _i, _l, _f, _f, _p], _i),
     "ia2p_inpaint_blend": ([_p, _p, _p, _p, _p, _l, _l, _l, _f, _f, _p], _i),
     "ia2p_polar_workspace_bytes": ([], _l),

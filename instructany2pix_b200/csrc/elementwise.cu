@@ -42,20 +42,34 @@ template <> __device__ __forceinline__ void store8<__half>(__half* p, const floa
   *reinterpret_cast<uint4*>(p) = a;
 }
 
+// v rounded to T's precision and back (what a later load of a stored T reads)
+template <typename T> __device__ __forceinline__ float round_to(float v);
+template <> __device__ __forceinline__ float round_to<float>(float v) { return v; }
+template <> __device__ __forceinline__ float round_to<__nv_bfloat16>(float v) { return __bfloat162float(__float2bfloat16_rn(v)); }
+template <> __device__ __forceinline__ float round_to<__half>(float v) { return __half2float(__float2half_rn(v)); }
+
 // ---------------------------------------------------------------- CFG + DDIM (one pass over the latents)
 // VEC = true: 8 elements per thread and iteration through 128-bit loads / stores; VEC = false: scalar fallback for unaligned or
 // ragged sizes.  total = batch * n; eps_u at [i], eps_c at [total + i].
 // ROWS = true: the guidance scale of sample i / n is g_rows[i / n] (one request per batch row); the VEC variant needs n % 8 == 0,
 // so the eight elements of a thread belong to one sample and one load serves them.  ROWS = false compiles to the scalar-g kernel.
-template <typename TE, typename TX, typename TI, bool VEC, bool ROWS>
+// COEF = true (with ROWS): c_x and c_e are per row too (cx_rows / ce_rows), and x_in2 is the NEXT UNet input of the batch rows
+// (not duplicated): x_in2[i] = s_rows[row] * x_out[i], with x_out[i] read back at TX precision -- bitwise axpby(x_out, x_out, s, 0)
+// for finite values.  The arithmetic of x_out is the scalar kernel's, so row b is bitwise the scalar kernel at that row's values.
+template <typename TE, typename TX, typename TI, bool VEC, bool ROWS, bool COEF = false>
 __global__ void cfg_ddim_kernel(const TE* __restrict__ eps2, const TX* __restrict__ x, TX* __restrict__ x_out,
                                 TI* __restrict__ x_in2, long long total, float g_scalar, float cx, float ce,
-                                const float* __restrict__ g_rows, long long n) {
+                                const float* __restrict__ g_rows, long long n, const float* __restrict__ cx_rows,
+                                const float* __restrict__ ce_rows, const float* __restrict__ s_rows) {
   pdl_launch_dependents();   // programmatic dependent launch: see common.cuh
   pdl_wait();
   constexpr int W = VEC ? 8 : 1;
   for (long long i = (blockIdx.x * (long long)blockDim.x + threadIdx.x) * W; i < total; i += (long long)gridDim.x * blockDim.x * W) {
     const float g = ROWS ? __ldg(g_rows + i / n) : g_scalar;
+    if constexpr (COEF) {
+      cx = __ldg(cx_rows + i / n);
+      ce = __ldg(ce_rows + i / n);
+    }
     if constexpr (VEC) {
       float eu[8], ec[8], xv[8], v[8];
       load8(eps2 + i, eu);
@@ -64,7 +78,14 @@ __global__ void cfg_ddim_kernel(const TE* __restrict__ eps2, const TX* __restric
 #pragma unroll
       for (int j = 0; j < 8; ++j) v[j] = cx * xv[j] + ce * (eu[j] + g * (ec[j] - eu[j]));
       store8(x_out + i, v);
-      if (x_in2 != nullptr) {
+      if constexpr (COEF) {
+        if (x_in2 != nullptr) {
+          const float s = __ldg(s_rows + i / n);
+#pragma unroll
+          for (int j = 0; j < 8; ++j) v[j] = s * round_to<TX>(v[j]);
+          store8(x_in2 + i, v);
+        }
+      } else if (x_in2 != nullptr) {
         store8(x_in2 + i, v);
         store8(x_in2 + total + i, v);
       }
@@ -72,7 +93,9 @@ __global__ void cfg_ddim_kernel(const TE* __restrict__ eps2, const TX* __restric
       const float eu = load_as_float(eps2 + i), ec = load_as_float(eps2 + total + i);
       const float v = cx * load_as_float(x + i) + ce * (eu + g * (ec - eu));
       store_from_float(x_out + i, v);
-      if (x_in2 != nullptr) {
+      if constexpr (COEF) {
+        if (x_in2 != nullptr) store_from_float(x_in2 + i, __ldg(s_rows + i / n) * round_to<TX>(v));
+      } else if (x_in2 != nullptr) {
         store_from_float(x_in2 + i, v);
         store_from_float(x_in2 + total + i, v);
       }
@@ -98,6 +121,39 @@ __global__ void axpby_kernel(const TE* __restrict__ eps, const TX* __restrict__ 
       store_from_float(out + i, cx * load_as_float(x + i) + ce * load_as_float(eps + i));
     }
   }
+}
+
+// ---------------------------------------------------------------- continuous batching: per-slot time-embedding rows
+// Slot s of an S-slot CFG batch owns UNet rows s (uncond) and S + s (cond).  tables[s] is [rows, 2 * sumC]: per step the blocked
+// rowbias of a CFG pair (block r = the [2, C_r] bias of ResnetBlock r); step[s] selects the row.  The kernel writes the blocked
+// [2S, C_r] blocks of the UNet batch and the slot's ncoef per-step coefficients to coef[j * S + s].  Grid (x, S, blocks).
+constexpr int kMaxRowbiasBlocks = 64;
+struct RowbiasBlocks { int lo[kMaxRowbiasBlocks + 1]; };
+
+__global__ void rowbias_gather_kernel(const float* __restrict__ tables, const float* __restrict__ coef_tables,
+                                      const int* __restrict__ step, float* __restrict__ rowbias, float* __restrict__ coef, int S,
+                                      int rows, int ncoef, RowbiasBlocks blk) {
+  pdl_launch_dependents();   // programmatic dependent launch: see common.cuh
+  pdl_wait();
+  const int s = blockIdx.y, r = blockIdx.z;
+  const int lo = blk.lo[r], C = blk.lo[r + 1] - lo, width = 2 * blk.lo[gridDim.z];
+  const int k = min(max(step[s], 0), rows - 1);
+  const float* src = tables + ((long long)s * rows + k) * width + 2LL * lo;
+  float* dst = rowbias + 2LL * S * lo;
+  for (int c = blockIdx.x * blockDim.x + threadIdx.x; c < C; c += gridDim.x * blockDim.x) {
+    dst[(long long)s * C + c] = src[c];
+    dst[(long long)(S + s) * C + c] = src[C + c];
+  }
+  if (blockIdx.x == 0 && r == 0 && threadIdx.x < ncoef)
+    coef[threadIdx.x * S + s] = coef_tables[((long long)s * rows + k) * ncoef + threadIdx.x];
+}
+
+// runs after the gather: every slot moves to its next row; the last row is the sentinel an idle slot stays on
+__global__ void step_advance_kernel(int* __restrict__ step, int S, int last) {
+  pdl_launch_dependents();
+  pdl_wait();
+  for (int s = threadIdx.x; s < S; s += blockDim.x)
+    if (step[s] < last) step[s] += 1;
 }
 
 __global__ void prior_step_kernel(const float* __restrict__ x0_pair, const float* __restrict__ x,
@@ -513,7 +569,7 @@ static int cfg_ddim_launch(const void* eps2, int eps_dtype, const void* x, void*
   DISPATCH_DTYPE(eps_dtype, TE, DISPATCH_DTYPE(x_dtype, TX, DISPATCH_DTYPE(xin_dtype, TI,                                       \
       (launch_pdl(cfg_ddim_kernel<TE, TX, TI, VEC_, ROWS_>, dim3(grid), dim3(256), 0, st, static_cast<const TE*>(eps2),         \
                   static_cast<const TX*>(x), static_cast<TX*>(x_out), static_cast<TI*>(x_in_next2), total, g, c_x, c_e, g_rows, \
-                  (long long)n)))))
+                  (long long)n, nullptr, nullptr, nullptr)))))
   if (g_rows == nullptr) {
     if (vec) { IA2P_CFG_DDIM(true, false); } else { IA2P_CFG_DDIM(false, false); }
   } else {
@@ -536,6 +592,63 @@ extern "C" int ia2p_cfg_ddim_step_rows(const void* eps2, int eps_dtype, const vo
   IA2P_REQUIRE(g != nullptr, IA2P_E_ARG, "cfg_ddim_step_rows: null guidance-scale array");
   IA2P_REQUIRE((reinterpret_cast<uintptr_t>(g) & 3) == 0, IA2P_E_ALIGN, "cfg_ddim_step_rows: g must be 4-byte aligned");
   return cfg_ddim_launch(eps2, eps_dtype, x, x_out, x_dtype, x_in_next2, xin_dtype, batch, n, 0.f, g, c_x, c_e, stream);
+}
+
+extern "C" int ia2p_cfg_step_coef_rows(const void* eps2, int eps_dtype, const void* x, void* x_out, int x_dtype,
+                                       void* x_in_next, int xin_dtype, int64_t batch, int64_t n, const float* g,
+                                       const float* c_x, const float* c_e, const float* s_in, void* stream) {
+  if (int e = check_device()) return e;
+  IA2P_REQUIRE(eps2 && x && x_out && batch > 0 && n > 0, IA2P_E_ARG, "cfg_step_coef_rows: null pointer or empty shape");
+  IA2P_REQUIRE(g && c_x && c_e, IA2P_E_ARG, "cfg_step_coef_rows: null coefficient array");
+  IA2P_REQUIRE((x_in_next == nullptr) == (s_in == nullptr), IA2P_E_ARG, "cfg_step_coef_rows: x_in_next and s_in go together");
+  auto al4 = [](const float* p) { return (reinterpret_cast<uintptr_t>(p) & 3) == 0; };
+  IA2P_REQUIRE(al4(g) && al4(c_x) && al4(c_e) && (s_in == nullptr || al4(s_in)), IA2P_E_ALIGN,
+               "cfg_step_coef_rows: coefficient arrays must be 4-byte aligned");
+  const long long total = batch * n;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (x_in_next == nullptr) xin_dtype = x_dtype;
+  auto esz = [](int dt) { return dt == IA2P_F32 ? 4ll : 2ll; };
+  auto al16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
+  // 128-bit path: as in cfg_ddim_launch, and every 8-element group lies inside one row
+  const bool vec = n % 8 == 0 && al16(eps2) && al16(x) && al16(x_out) && (x_in_next == nullptr || al16(x_in_next)) &&
+                   (total * esz(eps_dtype)) % 16 == 0;
+  const int grid = grid_for(vec ? total / 8 : total, 256);
+#define IA2P_CFG_COEF(VEC_)                                                                                                     \
+  DISPATCH_DTYPE(eps_dtype, TE, DISPATCH_DTYPE(x_dtype, TX, DISPATCH_DTYPE(xin_dtype, TI,                                       \
+      (launch_pdl(cfg_ddim_kernel<TE, TX, TI, VEC_, true, true>, dim3(grid), dim3(256), 0, st, static_cast<const TE*>(eps2),    \
+                  static_cast<const TX*>(x), static_cast<TX*>(x_out), static_cast<TI*>(x_in_next), total, 0.f, 1.f, 0.f, g,    \
+                  (long long)n, c_x, c_e, s_in)))))
+  if (vec) { IA2P_CFG_COEF(true); } else { IA2P_CFG_COEF(false); }
+#undef IA2P_CFG_COEF
+  IA2P_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int ia2p_rowbias_gather(const float* tables, const float* coef_tables, int* step, float* rowbias, float* coef,
+                                   int64_t slots, int64_t rows, const int64_t* block_lo, int64_t nblocks, int64_t ncoef,
+                                   void* stream) {
+  if (int e = check_device()) return e;
+  IA2P_REQUIRE(tables && coef_tables && step && rowbias && coef && block_lo, IA2P_E_ARG, "rowbias_gather: null pointer");
+  IA2P_REQUIRE(slots > 0 && slots <= 65535 && rows > 0 && ncoef > 0 && ncoef <= 256, IA2P_E_ARG,
+               "rowbias_gather: bad slots / rows / ncoef");
+  IA2P_REQUIRE(nblocks > 0 && nblocks <= kMaxRowbiasBlocks, IA2P_E_ARG, "rowbias_gather: 1..%d ResnetBlocks", kMaxRowbiasBlocks);
+  RowbiasBlocks blk;
+  int max_c = 0;
+  IA2P_REQUIRE(block_lo[0] == 0, IA2P_E_ARG, "rowbias_gather: the first block starts at column 0");
+  for (int r = 0; r <= nblocks; ++r) {
+    IA2P_REQUIRE(r == 0 || (block_lo[r] > block_lo[r - 1] && block_lo[r] < (1ll << 28)), IA2P_E_ARG,
+                 "rowbias_gather: block offsets must increase");
+    blk.lo[r] = (int)block_lo[r];
+    if (r && blk.lo[r] - blk.lo[r - 1] > max_c) max_c = blk.lo[r] - blk.lo[r - 1];
+  }
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const dim3 grid((max_c + 255) / 256, (unsigned)slots, (unsigned)nblocks);
+  IA2P_CUDA(launch_pdl(rowbias_gather_kernel, grid, dim3(256), 0, st, tables, coef_tables, (const int*)step, rowbias, coef,
+                       (int)slots, (int)rows, (int)ncoef, blk));
+  IA2P_LAUNCH_CHECK();
+  IA2P_CUDA(launch_pdl(step_advance_kernel, dim3(1), dim3(128), 0, st, step, (int)slots, (int)rows - 1));
+  IA2P_LAUNCH_CHECK();
+  return 0;
 }
 
 extern "C" int ia2p_axpby(const void* eps, int eps_dtype, const void* x, void* x_out, int x_dtype, int64_t n, float c_x,

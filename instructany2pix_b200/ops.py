@@ -175,6 +175,54 @@ def cfg_ddim_step(eps2, x, g, c_x, c_e, x_out=None, x_in_next2=None):
     return x_out
 
 
+def cfg_step_coef_rows(eps2, x, g, c_x, c_e, s_in=None, x_out=None, x_in_next=None):
+    """``cfg_ddim_step`` with every coefficient per row: x_out[b] = c_x[b]*x[b] + c_e[b]*(eps_u + g[b]*(eps_c - eps_u)).
+    ``g``, ``c_x``, ``c_e`` (and ``s_in``): contiguous fp32 CUDA tensors [batch], read when the kernel runs.  ``x_in_next``
+    [batch, ...] (with ``s_in``) receives s_in[b] * x_out[b], the row's next UNet input (not duplicated)."""
+    lib = _lib.load()
+    eps2, x = eps2.contiguous(), x.contiguous()
+    batch = x.shape[0]
+    n = x.numel() // batch
+    assert eps2.numel() == 2 * x.numel()
+    if (x_in_next is None) != (s_in is None):
+        raise ValueError("cfg_step_coef_rows: x_in_next and s_in go together")
+    g, c_x, c_e = (_row_scales(t, batch, f"cfg_step_coef_rows: {k}") for k, t in (("g", g), ("c_x", c_x), ("c_e", c_e)))
+    if s_in is not None:
+        s_in = _row_scales(s_in, batch, "cfg_step_coef_rows: s_in")
+        if x_in_next.shape != x.shape or not x_in_next.is_contiguous():
+            raise IA2PError(f"cfg_step_coef_rows: x_in_next must be a contiguous {tuple(x.shape)} tensor")
+    if x_out is None:
+        x_out = torch.empty_like(x)
+    _run(lib.ia2p_cfg_step_coef_rows, (eps2.data_ptr(), _DT[eps2.dtype], x.data_ptr(), x_out.data_ptr(), _DT[x.dtype],
+                                       _ptr(x_in_next), _DT[x_in_next.dtype] if x_in_next is not None else F32, batch, n,
+                                       g.data_ptr(), c_x.data_ptr(), c_e.data_ptr(), _ptr(s_in), _stream()), "cfg_step_coef_rows")
+    return x_out
+
+
+def rowbias_gather(tables, coef_tables, step, blocks, rowbias, coef):
+    """The step's blocked rowbias of an S-slot CFG batch from per-slot tables, then step[s] += 1 up to the last (sentinel) row.
+    tables fp32 [S, rows, 2 * sumC] (``time_rowbias_table(ts, pair, 2)`` rows), coef_tables fp32 [S, rows, ncoef], step int32 [S],
+    blocks: the ResnetBlocks' (lo, hi) column ranges (``prepare()["temb_slices"]``); rowbias fp32 [2 * S * sumC], coef fp32
+    [ncoef, S] are written."""
+    import ctypes
+    lib = _lib.load()
+    S, rows, width = tables.shape
+    ncoef = coef_tables.shape[-1]
+    lo = [int(a) for a, _ in blocks] + [int(blocks[-1][1])]
+    if width != 2 * lo[-1] or lo != sorted(lo) or lo[0] != 0 or any(int(a) != b for (a, _), b in zip(blocks[1:], (h for _, h in blocks))):
+        raise IA2PError(f"rowbias_gather: blocks {blocks} do not tile a table row of {width} = 2 * sumC columns")
+    for t, name, shape, dt in ((tables, "tables", (S, rows, width), torch.float32), (coef_tables, "coef_tables", (S, rows, ncoef), torch.float32),
+                               (step, "step", (S,), torch.int32), (rowbias, "rowbias", (S * width,), torch.float32),
+                               (coef, "coef", (ncoef, S), torch.float32)):
+        _need(t, dt, f"rowbias_gather: {name}")
+        if tuple(t.shape) != shape or not t.is_contiguous():
+            raise IA2PError(f"rowbias_gather: {name} must be a contiguous {shape} tensor, got {tuple(t.shape)}")
+    offs = (ctypes.c_int64 * len(lo))(*lo)
+    _run(lib.ia2p_rowbias_gather, (tables.data_ptr(), coef_tables.data_ptr(), step.data_ptr(), rowbias.data_ptr(), coef.data_ptr(),
+                                   S, rows, ctypes.addressof(offs), len(blocks), ncoef, _stream()), "rowbias_gather")
+    return rowbias
+
+
 def axpby(eps, x, c_x, c_e, out=None):
     """out = c_x*x + c_e*eps (inverse DDIM step, pnp_pipeline.py:73-85)."""
     lib = _lib.load()
