@@ -235,6 +235,11 @@ int ia2p_conv3x3_s2_padend_nhwc_bf16(const void* x, int64_t B, int64_t H, int64_
  * The input batch is read modulo `in_batch` (CFG duplication without cat([x]*2): custom_pipelines.py:332). */
 int ia2p_conv_in_nchw(const void* x, int x_dtype, int64_t in_batch, int64_t B, int64_t H, int64_t W, int64_t Cin,
                       const float* w, const float* bias, void* out, int out_dtype, int64_t Cout, void* stream);
+/* conv_in of the VAE encoder straight from an 8-bit image: x uint8 [B,H,W,Cin] is read as 2 * (q / 255) - 1 in fp32 (diffusers 0.26
+ * VaeImageProcessor.preprocess of a PIL image, each step rounded separately), the same 3x3 pad 1 conv as ia2p_conv_in_nchw follows;
+ * no fp32 image is stored.  -> NHWC (bf16|fp32). */
+int ia2p_conv_in_u8_nhwc(const void* x, int64_t B, int64_t H, int64_t W, int64_t Cin, const float* w, const float* bias,
+                         void* out, int out_dtype, int64_t Cout, void* stream);
 /* conv_out: 3x3 pad 1 conv from NHWC bf16 to NCHW (fp32|bf16|fp16), Cout in {3, 4, 8} (UNet eps, VAE image, VAE moments).
  * w fp32 [Cout,3,3,Cin] (K order ky,kx,cin). */
 int ia2p_conv_out_nhwc(const void* x, int64_t B, int64_t H, int64_t W, int64_t Cin,
@@ -244,6 +249,10 @@ int ia2p_conv_out_nhwc(const void* x, int64_t B, int64_t H, int64_t W, int64_t C
  * when it runs on the tensor cores (ia2p_conv3x3_nhwc_bf16 with the output channels zero-padded to 32): [3P] UNet conv_out
  * (4 eps channels), VAE decoder conv_out (3) / encoder conv_out (8). */
 int ia2p_nhwc_prefix_to_nchw(const float* x, int64_t ld, float* out, int64_t B, int64_t HW, int64_t C, void* stream);
+/* The same three leading channels as an 8-bit image out uint8 [B,H,W,3]: q = round_half_even(clamp(v / 2 + 0.5, 0, 1) * 255) in
+ * fp32, bit for bit diffusers 0.26's VaeImageProcessor.postprocess(output_type="pil") (denormalize, then numpy_to_pil); NaN -> 0.
+ * B*HW % 16 == 0, ld % 4 == 0, 16-byte aligned x and out.  Replaces the NCHW copy when the caller wants 8-bit images. */
+int ia2p_nhwc_prefix_to_u8_image(const float* x, int64_t ld, void* out, int64_t B, int64_t HW, void* stream);
 
 /* 1x1 conv over <= 8 channels, NCHW fp32 -> NCHW fp32: out = scale * (w x) + bias.  Replaces [3P] AutoencoderKL.post_quant_conv
  * / quant_conv with the latent (un)scaling of ddim/sdxl_pipeline.py:866 and pnp_pipeline.py:204 folded into `scale`. */

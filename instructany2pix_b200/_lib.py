@@ -55,6 +55,8 @@ SIGNATURES = {
     "ia2p_conv_in_nchw": ([_p, _i, _l, _l, _l, _l, _l, _p, _p, _p, _i, _l, _p], _i),
     "ia2p_conv_out_nhwc": ([_p, _l, _l, _l, _l, _p, _p, _p, _i, _l, _p], _i),
     "ia2p_nhwc_prefix_to_nchw": ([_p, _l, _p, _l, _l, _l, _p], _i),
+    "ia2p_conv_in_u8_nhwc": ([_p, _l, _l, _l, _l, _p, _p, _p, _i, _l, _p], _i),
+    "ia2p_nhwc_prefix_to_u8_image": ([_p, _l, _p, _l, _l, _p], _i),
     "ia2p_conv1x1_nchw_small": ([_p, _p, _p, _p, _l, _l, _l, _l, _f, _p], _i),
     "ia2p_softmax_rows_f32_bf16": ([_p, _l, _p, _l, _l, _l, _f, _p], _i),
     "ia2p_flash_self_attn_bf16": ([_p, _p, _p, _l, _p, _l, _l, _l, _i, _f, _p], _i),

@@ -309,6 +309,21 @@ __global__ void cast_bf16_kernel(const T* __restrict__ x, uint4* __restrict__ y,
 // Block = 64 output pixels: weights transposed to smem [K][Cout], the 64 input patches to smem [64][K]; each thread
 // produces channel quads (float4 weight reads conflict-free, patch reads broadcast), stores are fully coalesced.
 constexpr int kConvInTile = 64;
+
+// Input element (b, ci, iy, ix) of conv_in: NCHW fp32 | bf16 | fp16 latents ...
+template <typename TX>
+__device__ __forceinline__ float conv_in_input(const TX* x, long long b, int ci, int iy, int ix, int H, int W, int Cin) {
+  return load_as_float(x + ((b * Cin + ci) * H + iy) * (long long)W + ix);
+}
+// ... or an 8-bit NHWC image, mapped to [-1, 1] as diffusers 0.26's VaeImageProcessor.preprocess does it for a PIL image:
+// pil_to_numpy (np.float32(q) / 255) then normalize (2 x - 1), each step one correctly rounded fp32 operation (the __f*_rn
+// intrinsics are never contracted into an FMA).  The fp32 image exists only in the CTA's shared-memory patch.
+template <>
+__device__ __forceinline__ float conv_in_input<uint8_t>(const uint8_t* x, long long b, int ci, int iy, int ix, int H, int W, int Cin) {
+  const float q = (float)x[((b * H + iy) * (long long)W + ix) * Cin + ci];
+  return __fsub_rn(__fmul_rn(2.0f, __fdiv_rn(q, 255.0f)), 1.0f);
+}
+
 template <typename TX, typename TO>
 __global__ void __launch_bounds__(256)
 conv_in_kernel(const TX* __restrict__ x, long long in_batch, long long B, int H, int W, int Cin,
@@ -338,7 +353,7 @@ conv_in_kernel(const TX* __restrict__ x, long long in_batch, long long B, int H,
         const long long b = pix / ((long long)W * H);
         const int iy = yy + tap / 3 - 1, ix = xx + tap % 3 - 1;
         if (iy >= 0 && iy < H && ix >= 0 && ix < W)
-          v = load_as_float(x + (((b % in_batch) * Cin + ci) * H + iy) * (long long)W + ix);
+          v = conv_in_input(x, b % in_batch, ci, iy, ix, H, W, Cin);
       }
       sp[i] = v;
     }
@@ -472,6 +487,40 @@ __global__ void nhwc_prefix_to_nchw_kernel(const float* __restrict__ x, long lon
       v[4] = v1.x; v[5] = v1.y; v[6] = v1.z; v[7] = v1.w;
     }
     for (int c = 0; c < C; ++c) out[(b * C + c) * hw + p] = v[c];
+  }
+}
+
+// The decoder's image as 8 bits, what diffusers 0.26's VaeImageProcessor.postprocess(output_type="pil") hands out:
+// denormalize ((v / 2 + 0.5).clamp(0, 1)) then numpy_to_pil ((img * 255).round().astype("uint8")), all in fp32.  Every step is
+// one correctly rounded fp32 operation (__fmul_rn / __fadd_rn are never contracted into an FMA; v / 2 == v * 0.5 exactly) and
+// the conversion rounds half to even like np.round.  Non-finite inputs: +inf -> 255, -inf -> 0, NaN -> 0 (fmaxf returns the
+// non-NaN operand; numpy's NaN -> uint8 cast is undefined, and gives 0 on x86).
+__device__ __forceinline__ uint32_t image_u8(float v) {
+  const float c = fminf(fmaxf(__fadd_rn(__fmul_rn(v, 0.5f), 0.5f), 0.f), 1.f);
+  return __float2uint_rn(__fmul_rn(c, 255.0f));
+}
+
+// out[b, y, x, c] = image_u8(x[(b*hw + p) * ld + c]), c < 3: the leading three channels of the decoder conv_out's NHWC fp32 tensor
+// (output channels zero-padded to 32) as a uint8 [B, H, W, 3] image.  Thread = 16 pixels: sixteen 16-byte loads, the 48 result
+// bytes assembled in registers and written with three 16-byte stores.
+__global__ void nhwc_prefix_to_u8_image_kernel(const float* __restrict__ x, long long ld, uint4* __restrict__ out, long long ngroups) {
+  pdl_launch_dependents();
+  pdl_wait();
+  for (long long g = blockIdx.x * (long long)blockDim.x + threadIdx.x; g < ngroups; g += (long long)gridDim.x * blockDim.x) {
+    const float* p = x + g * 16 * ld;
+    float4 v[16];
+#pragma unroll
+    for (int j = 0; j < 16; ++j) v[j] = __ldg(reinterpret_cast<const float4*>(p + j * ld));
+    uint32_t w[12] = {};
+#pragma unroll
+    for (int j = 0; j < 16; ++j) {
+      const uint32_t q[3] = {image_u8(v[j].x), image_u8(v[j].y), image_u8(v[j].z)};
+#pragma unroll
+      for (int c = 0; c < 3; ++c) w[(3 * j + c) >> 2] |= q[c] << (8 * ((3 * j + c) & 3));
+    }
+    out[3 * g] = make_uint4(w[0], w[1], w[2], w[3]);
+    out[3 * g + 1] = make_uint4(w[4], w[5], w[6], w[7]);
+    out[3 * g + 2] = make_uint4(w[8], w[9], w[10], w[11]);
   }
 }
 
@@ -744,20 +793,18 @@ extern "C" int ia2p_cast_to_bf16(const void* x, int x_dtype, void* y, int64_t n,
   return 0;
 }
 
-extern "C" int ia2p_conv_in_nchw(const void* x, int x_dtype, int64_t in_batch, int64_t B, int64_t H, int64_t W, int64_t Cin,
-                                 const float* w, const float* bias, void* out, int out_dtype, int64_t Cout, void* stream) {
-  if (int e = check_device()) return e;
-  IA2P_REQUIRE(x && w && out && B > 0 && in_batch > 0 && H > 0 && W > 0, IA2P_E_ARG, "conv_in: bad arguments");
-  IA2P_REQUIRE(out_dtype == IA2P_BF16 || out_dtype == IA2P_F32, IA2P_E_ARG, "conv_in: out_dtype must be bf16 or f32");
-  // Cin = 4: latents; 8 / 9: inpainting UNets (latents + mask + masked-image latents, [3P] StableDiffusionXLInpaintPipeline)
-  IA2P_REQUIRE(Cin >= 1 && Cin <= 16 && Cout % 8 == 0 && Cout <= 640, IA2P_E_SHAPE, "conv_in: Cin<=16, Cout%%8==0, Cout<=640 required");
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const long long npix = B * H * W;
-  const size_t smem = (size_t)Cin * 9 * (Cout + kConvInTile) * sizeof(float);
-  const long long ntiles = (npix + kConvInTile - 1) / kConvInTile;
-  const long long resident = (long long)sm_count() * (smem <= 56 * 1024 ? 4 : (smem <= 100 * 1024 ? 2 : 1));
-  const unsigned grid = (unsigned)(ntiles < resident ? ntiles : resident);      // persistent: weights are staged once per CTA
-  IA2P_REQUIRE(smem <= 200 * 1024, IA2P_E_SHAPE, "conv_in: shared-memory footprint too large");
+// grid and shared memory of conv_in_kernel (persistent: weights are staged once per CTA); checks shared in the two entry points
+#define IA2P_CONV_IN_GEOMETRY()                                                                                          \
+  IA2P_REQUIRE(w && out && B > 0 && H > 0 && W > 0, IA2P_E_ARG, "conv_in: bad arguments");                               \
+  IA2P_REQUIRE(out_dtype == IA2P_BF16 || out_dtype == IA2P_F32, IA2P_E_ARG, "conv_in: out_dtype must be bf16 or f32");   \
+  IA2P_REQUIRE(Cin >= 1 && Cin <= 16 && Cout % 8 == 0 && Cout <= 640, IA2P_E_SHAPE, "conv_in: Cin<=16, Cout%%8==0, Cout<=640 required"); \
+  cudaStream_t st = static_cast<cudaStream_t>(stream);                                                                   \
+  const long long npix = B * H * W;                                                                                      \
+  const size_t smem = (size_t)Cin * 9 * (Cout + kConvInTile) * sizeof(float);                                            \
+  const long long ntiles = (npix + kConvInTile - 1) / kConvInTile;                                                       \
+  const long long resident = (long long)sm_count() * (smem <= 56 * 1024 ? 4 : (smem <= 100 * 1024 ? 2 : 1));            \
+  const unsigned grid = (unsigned)(ntiles < resident ? ntiles : resident);                                               \
+  IA2P_REQUIRE(smem <= 200 * 1024, IA2P_E_SHAPE, "conv_in: shared-memory footprint too large")
 #define IA2P_CONV_IN(TX_, TO_)                                                                                           \
   do {                                                                                                                   \
     if (smem > 48 * 1024)                                                                                                \
@@ -765,15 +812,38 @@ extern "C" int ia2p_conv_in_nchw(const void* x, int x_dtype, int64_t in_batch, i
     launch_pdl(conv_in_kernel<TX_, TO_>, dim3(grid), dim3(256), smem, st, static_cast<const TX_*>(x), in_batch, B, (int)H, (int)W, (int)Cin, w, \
                                                       bias, static_cast<TO_*>(out), (int)Cout);                         \
   } while (0)
+
+extern "C" int ia2p_conv_in_nchw(const void* x, int x_dtype, int64_t in_batch, int64_t B, int64_t H, int64_t W, int64_t Cin,
+                                 const float* w, const float* bias, void* out, int out_dtype, int64_t Cout, void* stream) {
+  if (int e = check_device()) return e;
+  IA2P_REQUIRE(x && in_batch > 0, IA2P_E_ARG, "conv_in: bad arguments");
+  // Cin = 4: latents; 8 / 9: inpainting UNets (latents + mask + masked-image latents, [3P] StableDiffusionXLInpaintPipeline)
+  IA2P_CONV_IN_GEOMETRY();
   if (out_dtype == IA2P_BF16) {
     DISPATCH_DTYPE(x_dtype, TX, IA2P_CONV_IN(TX, __nv_bfloat16));
   } else {
     DISPATCH_DTYPE(x_dtype, TX, IA2P_CONV_IN(TX, float));
   }
-#undef IA2P_CONV_IN
   IA2P_LAUNCH_CHECK();
   return 0;
 }
+
+extern "C" int ia2p_conv_in_u8_nhwc(const void* x, int64_t B, int64_t H, int64_t W, int64_t Cin, const float* w, const float* bias,
+                                    void* out, int out_dtype, int64_t Cout, void* stream) {
+  if (int e = check_device()) return e;
+  IA2P_REQUIRE(x, IA2P_E_ARG, "conv_in_u8: bad arguments");
+  const long long in_batch = B;
+  IA2P_CONV_IN_GEOMETRY();
+  if (out_dtype == IA2P_BF16) {
+    IA2P_CONV_IN(uint8_t, __nv_bfloat16);
+  } else {
+    IA2P_CONV_IN(uint8_t, float);
+  }
+  IA2P_LAUNCH_CHECK();
+  return 0;
+}
+#undef IA2P_CONV_IN
+#undef IA2P_CONV_IN_GEOMETRY
 
 extern "C" int ia2p_conv_out_nhwc(const void* x, int64_t B, int64_t H, int64_t W, int64_t Cin, const float* w,
                                   const float* bias, void* out, int out_dtype, int64_t Cout, void* stream) {
@@ -812,6 +882,19 @@ extern "C" int ia2p_nhwc_prefix_to_nchw(const float* x, int64_t ld, float* out, 
   IA2P_REQUIRE(ld % 4 == 0 && ld >= 8 && (reinterpret_cast<uintptr_t>(x) & 15) == 0, IA2P_E_ALIGN, "nhwc_prefix_to_nchw: ld %% 4 == 0, ld >= 8, 16-byte base");
   IA2P_CUDA(launch_pdl(nhwc_prefix_to_nchw_kernel, dim3(grid_for(B * HW, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream), x, (long long)ld,
                        out, (long long)B, (long long)HW, (int)C));
+  IA2P_LAUNCH_CHECK();
+  return 0;
+}
+
+extern "C" int ia2p_nhwc_prefix_to_u8_image(const float* x, int64_t ld, void* out, int64_t B, int64_t HW, void* stream) {
+  if (int e = check_device()) return e;
+  IA2P_REQUIRE(x && out && B > 0 && HW > 0, IA2P_E_ARG, "nhwc_prefix_to_u8_image: bad arguments");
+  IA2P_REQUIRE((B * HW) % 16 == 0, IA2P_E_SHAPE, "nhwc_prefix_to_u8_image: B*HW = %lld must be a multiple of 16", (long long)(B * HW));
+  IA2P_REQUIRE(ld % 4 == 0 && ld >= 4 && (reinterpret_cast<uintptr_t>(x) & 15) == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0,
+               IA2P_E_ALIGN, "nhwc_prefix_to_u8_image: ld %% 4 == 0 and 16-byte aligned bases required");
+  const long long ngroups = B * HW / 16;
+  IA2P_CUDA(launch_pdl(nhwc_prefix_to_u8_image_kernel, dim3(grid_for(ngroups, 256)), dim3(256), 0, static_cast<cudaStream_t>(stream), x,
+                       (long long)ld, static_cast<uint4*>(out), ngroups));
   IA2P_LAUNCH_CHECK();
   return 0;
 }

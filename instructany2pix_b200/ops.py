@@ -643,6 +643,44 @@ def conv_out_tc(x, w32, b32, cout):
     return out
 
 
+def conv_in_u8(x, w, bias, out_dtype=torch.bfloat16):
+    """conv_in straight from an 8-bit image: x uint8 [B, H, W, Cin] is read as ``2 * (q / 255) - 1`` in fp32 (diffusers'
+    ``VaeImageProcessor.preprocess`` of a PIL image) -> NHWC (bf16|fp32); w fp32 [Cout, Cin, 3, 3]."""
+    lib = _lib.load()
+    _need(x, torch.uint8, "x", 4)
+    x = x.contiguous()
+    B, H, W, cin = x.shape
+    w, bias = _f32(w, "w"), _f32(bias, "bias")
+    if w.shape[1] != cin:
+        raise IA2PError(f"conv_in_u8: image has {cin} channels, the weights expect {w.shape[1]}")
+    cout = w.shape[0]
+    out = torch.empty(B, H, W, cout, device=x.device, dtype=out_dtype)
+    global _BYTES
+    _BYTES = x.numel() + out.numel() * out.element_size() + 4.0 * w.numel()
+    _run(lib.ia2p_conv_in_u8_nhwc, (x.data_ptr(), B, H, W, cin, w.data_ptr(), _ptr(bias), out.data_ptr(), _DT[out_dtype], cout,
+                                        _stream()), "conv_in_u8")
+    return out
+
+
+def image_u8(y):
+    """The first three channels of an NHWC fp32 tensor y [B, H, W, C >= 4] (C % 4 == 0) as an 8-bit image uint8 [B, H, W, 3]:
+    ``round_half_even(clamp(v / 2 + 0.5, 0, 1) * 255)``, bit for bit diffusers' ``postprocess(output_type="pil")``; NaN -> 0."""
+    lib = _lib.load()
+    _need(y, torch.float32, "y", 4)
+    y = y.contiguous()
+    B, H, W, ld = y.shape
+    out = torch.empty(B, H, W, 3, device=y.device, dtype=torch.uint8)
+    global _BYTES
+    _BYTES = 16.0 * B * H * W + out.numel()
+    _run(lib.ia2p_nhwc_prefix_to_u8_image, (y.data_ptr(), ld, out.data_ptr(), B, H * W, _stream()), "image_u8")
+    return out
+
+
+def conv_out_u8(x, w32, b32):
+    """``conv_out_tc`` of the VAE decoder with its image written as uint8 [B, H, W, 3] (``image_u8``) instead of fp32 NCHW."""
+    return image_u8(conv3x3(x, w32, 32, bias=b32, out_dtype=torch.float32))
+
+
 def conv1x1_nchw_small(x, w, bias, scale=1.0):
     """1x1 conv over <= 8 channels, NCHW fp32 -> NCHW fp32: scale * (w x) + bias (VAE post_quant_conv / quant_conv)."""
     lib = _lib.load()

@@ -215,8 +215,10 @@ class B200Sampler:
 
     # ------------------------------------------------------------------ DDIM inversion (batch B, no CFG)
     @torch.no_grad()
-    def invert(self, latents, ctx, added_cond_kwargs, num_inference_steps=50, trace=None):
-        s = self.scheduler
+    def invert(self, latents, ctx, added_cond_kwargs, num_inference_steps=50, trace=None, scheduler=None):
+        """DDIM inversion on ``scheduler`` (default: the sampler's own).  The reference inverts with a DDIM scheduler of its own
+        whatever scheduler generates (pnp_pipeline.py:133); the graph cache is the sampler's either way."""
+        s = scheduler or self.scheduler
         s.set_timesteps(num_inference_steps)
         B = latents.shape[0]
         ts = list(reversed(s.timesteps.tolist()))

@@ -229,9 +229,15 @@ class B200VAE(nn.Module):
 
     # ------------------------------------------------------------------ decode (sdxl_pipeline.py:859-871)
     @torch.no_grad()
-    def decode(self, latents, scaled=True):
+    def decode(self, latents, scaled=True, output="float"):
         """latents (B,4,L,L) as the sampler returns them -> images (B,3,8L,8L) fp32, nominal range [-1, 1].
-        ``scaled=True`` folds the reference's ``latents / scaling_factor`` into post_quant_conv."""
+        ``scaled=True`` folds the reference's ``latents / scaling_factor`` into post_quant_conv.
+        ``output="u8"``: 8-bit images uint8 (B,8L,8L,3) instead, bit for bit what diffusers' ``postprocess(output_type="pil")``
+        makes of the fp32 images (``ops.image_u8``), written by the last kernel of the decoder."""
+        if output not in ("float", "u8"):
+            raise ValueError(f"output: 'float' or 'u8', got {output!r}")
+        if output == "u8" and self.config.out_channels != 3:
+            raise ValueError(f"output='u8' needs a 3-channel image, the decoder has {self.config.out_channels}")
         P, cfg = self.prepare(), self.config
         G = cfg.norm_num_groups
         z = ops.conv1x1_nchw_small(latents.to(self.device, torch.float32), self.post_quant_conv.weight, self.post_quant_conv.bias,
@@ -245,16 +251,25 @@ class B200VAE(nn.Module):
                 q = P[f"decoder.up_blocks.{i}.upsamplers.0"]
                 x = ops.conv_up2x(ops.to_bf16(x), q["w4"], q["w"].shape[0], bias=q["b"], want_colstats=True)   # Upsample2D folded
         h = ops.groupnorm(x, None, *P["decoder.norm_out"], G, 1e-6, True)
+        if output == "u8":
+            return ops.conv_out_u8(h, *P["decoder.conv_out"])
         return ops.conv_out_tc(h, *P["decoder.conv_out"], cfg.out_channels)
 
     # ------------------------------------------------------------------ encode (pnp_pipeline.py:195-204)
     @torch.no_grad()
     def encode(self, images, noise=None, generator=None, sample=True, scaled=True):
         """images (B,3,H,W) in [-1, 1] -> latents (B,4,H/8,W/8) fp32 = ``latent_dist.sample() * scaling_factor``
-        (``sample=False``: the mode).  ``noise`` may be supplied for parity tests; ``generator`` may be one generator per image."""
+        (``sample=False``: the mode).  ``noise`` may be supplied for parity tests; ``generator`` may be one generator per image.
+        ``images`` may also be 8-bit, uint8 (B,H,W,3): the first conv reads them as ``2 * (q / 255) - 1`` (diffusers'
+        ``preprocess`` of a PIL image) without storing an fp32 image."""
         P, cfg = self.prepare(), self.config
         G = cfg.norm_num_groups
-        x = ops.conv_in(images.to(self.device, torch.float32), *P["encoder.conv_in"], out_dtype=torch.float32)
+        if images.dtype == torch.uint8:
+            if images.ndim != 4 or images.shape[-1] != cfg.in_channels:
+                raise ValueError(f"an 8-bit image is (B, H, W, {cfg.in_channels}), got {tuple(images.shape)}")
+            x = ops.conv_in_u8(images.to(self.device), *P["encoder.conv_in"], out_dtype=torch.float32)
+        else:
+            x = ops.conv_in(images.to(self.device, torch.float32), *P["encoder.conv_in"], out_dtype=torch.float32)
         for i, blk in enumerate(self.encoder.down_blocks):
             for j in range(len(blk.resnets)):
                 x = self._res(P, f"encoder.down_blocks.{i}.resnets.{j}", x)
